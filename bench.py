@@ -2,6 +2,7 @@
 """bench.py -- aggregate env-steps/s of the batched ECS step engine.
 
     python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" = one pass of the simulator's step task graph over all worlds
 (MWCudaExecutor::run equivalent).  One process per GPU (torchrun for N>1);
@@ -22,6 +23,14 @@ line on rank 0.
             the actions H2D from pinned memory and reads rewards+dones back D2H.
   roofline  dominant node of the step (per-node CUDA-event timing inside this
             process via mb2_profile_nodes) vs MEASURED_PEAKS.json hbm_gbs.
+  --dump-outputs DIR
+            after the K timed steps, rank 0 writes the exported columns of its
+            worlds as they stand after the last timed step (what run() hands a
+            caller, plus the rendered views) to DIR/<name>.npy: float32 columns
+            as they are, integer columns as float64 (exact), RGBA8 as float32.
+            A column over its share of 64 MiB is a fixed seeded sample of its
+            rows.  Actions and world seeds are fixed, so two builds given the
+            same arguments can be compared output for output.
   cpu_baseline / --impl reference
             the reference's own CPU backend (oracle/_ref, built from the
             reference sources) running the same fixture on the host cores.
@@ -117,6 +126,29 @@ class ClockSampler:
 
 
 N_ACT = 16   # length of the action cycle both arms replay
+DUMP_BYTES = 64 << 20   # all dumped columns together
+
+
+def dump_outputs(ex, desc, W, cfg, render, out_dir):
+    """Writes the exported columns (and rendered views) to out_dir/<name>.npy; see --dump-outputs."""
+    cols = [(s.name, s.slot, s.dtype, ((ex.exportedNumRows(s.slot) if s.dynamic else W),) + s.per_world)
+            for s in desc.outputs]
+    if render:
+        res, views = int(cfg.get("resolution", 64)), ex.exportedNumRows(14)
+        cols.append(("depth", 14, "float32", (views, res, res)))
+        if cfg.get("rgbd"):
+            cols.append(("rgba", 13, "uint8", (views, res, res, 4)))
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // len(cols)
+    for name, slot, dtype, shape in cols:
+        arr = ex.tensor(slot, dtype, shape).cpu().numpy() if shape[0] else np.zeros(shape, dtype)
+        arr = arr.astype(np.float64 if np.issubdtype(arr.dtype, np.integer) and arr.itemsize > 1
+                         else np.float32)
+        row_bytes = max(arr[:1].nbytes, 1)
+        if arr.nbytes > cap:
+            keep = cap // row_bytes
+            arr = arr[np.sort(np.random.default_rng(0).choice(len(arr), size=keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def make_actions(desc, sim, W, steps, seed):
@@ -222,6 +254,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--gather", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: NVLink peer-store gather kernel (default) or one packed NCCL all_gather per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (rank 0's worlds)")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
     if args.worlds:
@@ -431,6 +465,9 @@ def main():
     if sampler:
         sampler.start()
     total_ms, rank_stats = timed(host_io=False)
+    if args.dump_outputs and rank == 0:
+        torch.cuda.synchronize()
+        dump_outputs(ex, desc, W, cfg, render_graph is not None, args.dump_outputs)
     e2e_ms, e2e_rank_stats = timed(host_io=True)
     if world_size > 1:
         gather_drain()

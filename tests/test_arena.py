@@ -16,7 +16,7 @@ import pytest
 
 from oracle import runner
 from sims import SIMS
-from trace_utils import assert_traces_equal, load_golden, make_inputs, rollout_gpu
+from trace_utils import assert_matches_digest_golden, assert_traces_equal, load_golden, make_inputs, rollout_gpu
 
 EXACT = os.environ.get("MADRONA_B200_FAST_MATH", "0") != "1"
 CFG = {"episode_len": 90, "seed": 17}
@@ -87,11 +87,10 @@ def test_independent_nodes_become_graph_branches(monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("arena"), reason="oracle/_ref not built")
 def test_gpu_matches_live_reference_many_worlds():
+    # the reference CPU backend's trace is stored as a digest golden (tests/golden/make_golden.py)
     W, steps = 160, 150
     cfg = {"episode_len": 60, "seed": 4000}
     ins = make_inputs("arena", W, steps, seed=21)
-    ref, _ = runner.run_reference(SIMS["arena"], W, steps, ins, cfg, workers=4)
     got, _ = rollout_gpu("arena", W, steps, ins, cfg)
-    assert_traces_equal(got, ref, exact=EXACT, rtol=1e-4, atol=1e-5)
+    assert_matches_digest_golden(got, "arena_w160_s150_ref", ins, exact=EXACT, rtol=1e-4, atol=1e-5)

@@ -11,7 +11,7 @@ import pytest
 
 from oracle import runner
 from sims import SIMS
-from trace_utils import assert_traces_equal, load_golden, rollout_gpu
+from trace_utils import assert_matches_digest_golden, assert_traces_equal, load_golden, rollout_gpu
 
 EXACT = os.environ.get("MADRONA_B200_FAST_MATH", "0") != "1"
 CFG = {"seed": 3}
@@ -53,13 +53,12 @@ def test_gpu_matches_golden():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("balls"), reason="oracle/_ref not built")
 def test_gpu_matches_live_reference_many_worlds():
+    # the reference CPU backend's trace is stored as a digest golden (tests/golden/make_golden.py)
     W, steps = 400, 150
     cfg = {"seed": 7000}
-    ref, _ = runner.run_reference(SIMS["balls"], W, steps, {}, cfg, workers=4)
     got, _ = rollout_gpu("balls", W, steps, {}, cfg)
-    assert_traces_equal(got, ref, exact=EXACT, rtol=1e-4, atol=1e-5)
+    assert_matches_digest_golden(got, "balls_w400_s150_ref", {}, exact=EXACT, rtol=1e-4, atol=1e-5)
 
 
 # ---- build variant with 95 bodies per world (-DBALLS_MANY=1) ---------------------------------
@@ -87,12 +86,10 @@ def test_many_gpu_matches_golden(monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("balls_many"), reason="oracle/_ref not built")
 def test_many_gpu_matches_live_reference(monkeypatch):
     for k, v in MANY_ENV.items():
         monkeypatch.setenv(k, v)
     W, steps = 48, 80
     cfg = {"seed": 31000}
-    ref, _ = runner.run_reference(SIMS["balls_many"], W, steps, {}, cfg, workers=4)
     got, _ = rollout_gpu("balls_many", W, steps, {}, cfg)
-    assert_traces_equal(got, ref, exact=EXACT, rtol=1e-4, atol=1e-5)
+    assert_matches_digest_golden(got, "balls_many_w48_s80_ref", {}, exact=EXACT, rtol=1e-4, atol=1e-5)

@@ -7,7 +7,7 @@ import pytest
 
 from oracle import runner
 from sims import SIMS
-from trace_utils import load_golden as _load, make_inputs, rollout_gpu
+from trace_utils import assert_matches_digest_golden, load_golden as _load, make_inputs, rollout_gpu
 
 
 @pytest.mark.skipif(not runner.available("cartpole"), reason="oracle/_ref not built")
@@ -57,12 +57,10 @@ def test_gpu_matches_golden_bit_exact(name, cfg):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("cartpole"), reason="oracle/_ref not built")
 def test_gpu_matches_live_reference_baseline_config():
-    # BASELINE.json configs[0]: 256 worlds, 1000 steps, random actions
+    # BASELINE.json configs[0]: 256 worlds, 1000 steps, random actions; the reference CPU
+    # backend's trace of this run is stored as a digest golden (tests/golden/make_golden.py)
     W, steps = 256, 1000
     ins = make_inputs("cartpole", W, steps, seed=42)
-    ref, _ = runner.run_reference(SIMS["cartpole"], W, steps, ins, {}, workers=1)
     got, _ = rollout_gpu("cartpole", W, steps, ins, {})
-    for k in ref:
-        assert np.array_equal(got[k].view(np.uint32), ref[k].view(np.uint32)), k
+    assert_matches_digest_golden(got, "cartpole_w256_s1000_ref", ins)

@@ -1,12 +1,12 @@
 """BASELINE.json full-size configurations on the GPU, checked through
 size-independent properties (the reference CPU backend cannot run these sizes:
-its tmp allocator alone is 32 MiB per world)."""
+its tmp allocator alone is 32 MiB per world).  The reference runs of the first
+worlds are stored as digest goldens (tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
-from oracle import runner
 from sims import SIMS
-from trace_utils import make_inputs
+from trace_utils import assert_matches_digest_golden, make_inputs
 
 
 def _rollout_prefix(sim, W, steps, ins, cfg, keep_worlds, rows_per_world=None):
@@ -36,7 +36,6 @@ def _rollout_prefix(sim, W, steps, ins, cfg, keep_worlds, rows_per_world=None):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("room"), reason="oracle/_ref not built")
 def test_room_8192_worlds_prefix_equals_reference():
     # configs[1]: 8192 worlds / GPU.  Worlds are independent and seeded by their
     # index, so worlds [0, 64) of the 8192-world GPU run must equal a 64-world run
@@ -44,23 +43,18 @@ def test_room_8192_worlds_prefix_equals_reference():
     W, keep, steps = 8192, 64, 60
     cfg = {"episode_len": 40, "seed": 7}
     ins = make_inputs("room", keep, steps, seed=31)
-    ref, _ = runner.run_reference(SIMS["room"], keep, steps, ins, cfg, workers=4)
     got = _rollout_prefix("room", W, steps, ins, cfg, keep)
-    for k in got:
-        assert np.array_equal(got[k].view(np.uint32), ref[k].view(np.uint32)), k
+    assert_matches_digest_golden(got, "room_w64_s60_prefix_ref", ins)
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("gridworld"), reason="oracle/_ref not built")
 def test_gridworld_65536_worlds_prefix_equals_reference():
     # configs[4]: 65536 worlds / GPU (3 radix passes, multi-tile onesweep)
     W, keep, steps = 65536, 128, 60
     cfg = {"grid_size": 6, "episode_len": 25, "init_items": 8, "seed": 3}
     ins = make_inputs("gridworld", keep, steps, seed=13)
-    ref, _ = runner.run_reference(SIMS["gridworld"], keep, steps, ins, cfg, workers=4)
     got = _rollout_prefix("gridworld", W, steps, ins, cfg, keep)
-    for k in got:
-        assert np.array_equal(got[k], ref[k]), k
+    assert_matches_digest_golden(got, "gridworld_w128_s60_prefix_ref", ins)
 
 
 @pytest.mark.gpu
@@ -76,14 +70,11 @@ def test_room_8192_worlds_is_deterministic_and_finite():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("arena"), reason="oracle/_ref not built")
 def test_arena_4096_worlds_prefix_equals_reference():
     # configs[2]: 4096 worlds / GPU.  Worlds [0, 48) of the 4096-world GPU run must equal
     # a 48-world run of the reference CPU backend bit for bit (an episode reset inside).
     W, keep, steps = 4096, 48, 70
     cfg = {"episode_len": 45, "seed": 11}
     ins = make_inputs("arena", keep, steps, seed=77)
-    ref, _ = runner.run_reference(SIMS["arena"], keep, steps, ins, cfg, workers=4)
     got = _rollout_prefix("arena", W, steps, ins, cfg, keep)
-    for k in got:
-        assert np.array_equal(got[k].view(np.uint32), ref[k].view(np.uint32)), k
+    assert_matches_digest_golden(got, "arena_w48_s70_prefix_ref", ins)

@@ -1,9 +1,10 @@
 """GJK closest point (sphere - hull contacts): pins madrona_b200/device/madrona/gjk.hpp
 to the reference's src/physics/gjk.hpp + geo::hullClosestPointToOriginGJK.
 
-* oracle/gjk_probe.cpp is compiled against the reference (private header +
-  libmadrona_ref.a) and against the engine's header; the two binaries must print
-  identical bits: 900 sub-simplex solves, 1200 hull distance queries (a third of
+* oracle/gjk_probe.cpp compiled against the engine's header must print the bits
+  it printed compiled against the reference (private header + libmadrona_ref.a;
+  tests/golden holds the digest of that output and its known answers):
+  900 sub-simplex solves, 1200 hull distance queries (a third of
   them with the origin inside the hull);
 * the assertions of the reference's own tests (tests/gjk.cpp:18-47) are applied
   to both outputs.
@@ -11,21 +12,18 @@ to the reference's src/physics/gjk.hpp + geo::hullClosestPointToOriginGJK.
 import hashlib
 import os
 import struct
-import subprocess
 
 import pytest
 
+from trace_utils import build_engine_probe, reference_probe_output
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "gjk_probe_ref")
-MINE = os.path.join(ROOT, "oracle", "_ref", "gjk_probe_mine")
 GOLDEN = os.path.join(ROOT, "tests", "golden", "gjk_probe.sha256")
 
-needs_probes = pytest.mark.skipif(not (os.path.exists(REF) and os.path.exists(MINE)),
-                                  reason="oracle/_ref not built")
 
-
-def _run(path):
-    return subprocess.run([path], capture_output=True, text=True, check=True).stdout
+@pytest.fixture(scope="module")
+def mine(tmp_path_factory):
+    return build_engine_probe("gjk_probe_mine", tmp_path_factory.mktemp("probe"))
 
 
 def _f(hexbits):
@@ -40,20 +38,18 @@ def _tagged(text):
     return out
 
 
-@needs_probes
-def test_engine_header_matches_reference_bit_for_bit():
-    ref, mine = _run(REF), _run(MINE)
-    assert len(ref.splitlines()) > 10000
-    assert ref == mine
-    # the committed digest was produced by the reference build (tests/golden/make_golden.py)
-    if os.path.exists(GOLDEN):
-        assert hashlib.sha256(ref.encode()).hexdigest() == open(GOLDEN).read().strip()
+def test_engine_header_matches_reference_bit_for_bit(mine):
+    # the digest of the reference build's output (tests/golden/make_golden.py)
+    assert len(mine.splitlines()) > 10000
+    assert hashlib.sha256(mine.encode()).hexdigest() == open(GOLDEN).read().strip()
+    # its known answers, stored whole
+    ref_kat = reference_probe_output("gjk_probe_ref")
+    assert ref_kat.splitlines() == [ln for ln in mine.splitlines() if ln.startswith("kat_")]
 
 
-@needs_probes
-@pytest.mark.parametrize("binary", [REF, MINE], ids=["reference", "engine"])
-def test_reference_gjk_known_answers(binary):
-    vals = _tagged(_run(binary))
+@pytest.mark.parametrize("binary", ["reference", "engine"], ids=["reference", "engine"])
+def test_reference_gjk_known_answers(binary, mine):
+    vals = _tagged(reference_probe_output("gjk_probe_ref") if binary == "reference" else mine)
     # tests/gjk.cpp:18-32 Solve4SimplexDuplicatePoint
     assert vals["kat_dup_diff"][0] <= 1e-5
     # tests/gjk.cpp:34-47 Solve4SimplexAroundOrigin
@@ -62,8 +58,5 @@ def test_reference_gjk_known_answers(binary):
     assert len2 < 1e-5
 
 
-@pytest.mark.skipif(not os.path.exists(MINE), reason="oracle/_ref not built")
-def test_engine_header_against_committed_digest():
-    if not os.path.exists(GOLDEN):
-        pytest.skip("no committed digest")
-    assert hashlib.sha256(_run(MINE).encode()).hexdigest() == open(GOLDEN).read().strip()
+def test_engine_header_against_committed_digest(mine):
+    assert hashlib.sha256(mine.encode()).hexdigest() == open(GOLDEN).read().strip()

@@ -3,28 +3,29 @@ known-answer tests and headers.
 
 * reference KATs: tests/rand.cpp:131-141 (bits32 / sampleI32 upper limit),
   tests/math.cpp:23-48 (quaternion values, 1e-4);
-* header equivalence: oracle/kat_probe.cpp compiled against the reference
-  headers and against madrona_b200/device/madrona must print identical bits
-  (2500+ values: threefry streams, quaternion / matrix / AABB algebra);
+* header equivalence: oracle/kat_probe.cpp compiled against madrona_b200/device/madrona
+  must print the bits it printed compiled against the reference headers
+  (tests/golden/kat_probe_ref.txt.gz, 2500+ values: threefry streams,
+  quaternion / matrix / AABB algebra);
 * the numpy restatement (oracle/restate.py) must reproduce the same streams and
   the initial states the reference CPU backend produced in the golden traces.
 """
-import os
 import struct
-import subprocess
 
 import numpy as np
 import pytest
 
 from oracle import restate
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "kat_probe_ref")
-MINE = os.path.join(ROOT, "oracle", "_ref", "kat_probe_mine")
+from trace_utils import build_engine_probe, reference_probe_output
 
 
-def _run(path):
-    return subprocess.run([path], capture_output=True, text=True, check=True).stdout.splitlines()
+def _ref():
+    return reference_probe_output("kat_probe_ref").splitlines()
+
+
+@pytest.fixture(scope="module")
+def mine(tmp_path_factory):
+    return build_engine_probe("kat_probe_mine", tmp_path_factory.mktemp("probe")).splitlines()
 
 
 def _f(hexbits):
@@ -38,10 +39,9 @@ def test_restatement_known_answers():
     assert restate.sample_i32_biased(k, 0, 64) == 63
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built")
 def test_reference_headers_known_answers():
     lines = dict()
-    for ln in _run(REF):
+    for ln in _ref():
         tag, *vals = ln.split()
         lines.setdefault(tag, []).append(vals)
     assert lines["kat_bits32"][0][0] == "ffffffff"
@@ -55,16 +55,14 @@ def test_reference_headers_known_answers():
         assert np.allclose(got, q, atol=1e-4), (tag, got)
 
 
-@pytest.mark.skipif(not (os.path.exists(REF) and os.path.exists(MINE)), reason="oracle/_ref not built")
-def test_engine_headers_match_reference_headers_bit_for_bit():
-    ref, mine = _run(REF), _run(MINE)
+def test_engine_headers_match_reference_headers_bit_for_bit(mine):
+    ref = _ref()
     assert len(ref) > 2000
     assert ref == mine
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built")
 def test_restatement_matches_reference_streams():
-    lines = _run(REF)
+    lines = _ref()
     it = iter(lines)
     checked = 0
     for seed in range(4):

@@ -1,10 +1,10 @@
 """Physics asset pipeline (mb2_process_rigid_body_assets) against the reference's own
 RigidBodyAssets::processRigidBodyAssets (src/physics/physics_assets.cpp:1268, run by
-oracle/_ref/assets_probe_ref): half-edge numbering, face planes, AABBs and the mass
+oracle/assets_probe.cpp; its output is stored under tests/golden): half-edge numbering, face planes, AABBs and the mass
 properties (centre of mass, diagonalised inertia, inertia frame) must be bit-identical."""
+import hashlib
 import os
 import struct
-import subprocess
 import sys
 
 import numpy as np
@@ -16,7 +16,7 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 from sims.objects import orient_faces  # noqa: E402
 
-PROBE = os.path.join(ROOT, "oracle", "_ref", "assets_probe_ref")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "assets_probe_ref.npz")
 
 
 def _prism(n, sx=1.0, sy=1.0, sz=1.0, offset=(0, 0, 0)):
@@ -158,13 +158,17 @@ def _compare(mine, ref):
             assert a == b
 
 
-@pytest.mark.skipif(not os.path.exists(PROBE), reason="oracle/_ref/assets_probe_ref not built")
 def test_matches_reference_pipeline(tmp_path):
+    # the reference pipeline's output for _case() is stored in tests/golden/assets_probe_ref.npz
+    # (tests/golden/make_golden.py runs the probe)
     import madrona_b200 as mb
     hulls, objects = _case()
     inp, outp = str(tmp_path / "in.bin"), str(tmp_path / "out.bin")
     _write_probe_input(inp, hulls, objects)
-    subprocess.run([PROBE, inp, outp], check=True, timeout=120)
+    golden = np.load(GOLDEN)
+    assert hashlib.sha256(open(inp, "rb").read()).hexdigest() == str(golden["input_sha256"]), \
+        "the probe input differs from the one the golden output was made from"
+    golden["output"].tofile(outp)
     ref = _read_probe_output(outp)
     assets = mb.RigidBodyAssets(hulls, objects, gpu_id=-1)
     _compare(assets.host_arrays(), ref)

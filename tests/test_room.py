@@ -15,7 +15,8 @@ import pytest
 
 from oracle import runner
 from sims import SIMS
-from trace_utils import assert_traces_equal, load_golden, make_inputs, rollout_gpu
+from trace_utils import (assert_matches_digest_golden, assert_traces_equal, golden_path, load_golden,
+                         make_inputs, rollout_gpu)
 
 EXACT = os.environ.get("MADRONA_B200_FAST_MATH", "0") != "1"
 CFG = {"episode_len": 100, "seed": 21}
@@ -55,14 +56,13 @@ def test_gpu_matches_golden():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("room"), reason="oracle/_ref not built")
 def test_gpu_matches_live_reference_many_worlds():
+    # the reference CPU backend's trace is stored as a digest golden (tests/golden/make_golden.py)
     W, steps = 300, 130
     cfg = {"episode_len": 60, "seed": 1000}
     ins = make_inputs("room", W, steps, seed=9)
-    ref, _ = runner.run_reference(SIMS["room"], W, steps, ins, cfg, workers=4)
     got, _ = rollout_gpu("room", W, steps, ins, cfg)
-    assert_traces_equal(got, ref, exact=EXACT, rtol=1e-4, atol=1e-5)
+    assert_matches_digest_golden(got, "room_w300_s130_ref", ins, exact=EXACT, rtol=1e-4, atol=1e-5)
 
 
 GRAB_CFG = {"episode_len": 70, "seed": 5, "grab_period": 5}
@@ -70,11 +70,11 @@ GRAB_CFG = {"episode_len": 70, "seed": 5, "grab_period": 5}
 
 def test_grab_golden_has_joint_effects():
     W, steps, ins, outs = load_golden("room_grab_w3_s120")
-    base, _ = (runner.run_reference(SIMS["room"], W, steps, ins, {"episode_len": 70, "seed": 5}, workers=1)
-               if runner.available("room") else (None, None))
-    if base is not None:
-        diff = max(float(np.abs(a - b).max()) for a, b in zip(outs["body_pos"], base["body_pos"]))
-        assert diff > 0.1          # joints really moved cubes
+    # the reference CPU backend on the same inputs without grabbing (every tenth frame)
+    base = np.load(golden_path("room_nograb_w3_s120"))["body_pos"]
+    assert len(base) == len(outs["body_pos"][::10])
+    diff = max(float(np.abs(a - b).max()) for a, b in zip(outs["body_pos"][::10], base))
+    assert diff > 0.1          # joints really moved cubes
 
 
 @pytest.mark.gpu
@@ -87,11 +87,9 @@ def test_gpu_joints_match_golden():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("room"), reason="oracle/_ref not built")
 def test_gpu_joints_match_live_reference():
     W, steps = 200, 90
     cfg = {"episode_len": 50, "seed": 77, "grab_period": 3}
     ins = make_inputs("room", W, steps, seed=4)
-    ref, _ = runner.run_reference(SIMS["room"], W, steps, ins, cfg, workers=4)
     got, _ = rollout_gpu("room", W, steps, ins, cfg)
-    assert_traces_equal(got, ref, exact=EXACT, rtol=1e-4, atol=1e-5)
+    assert_matches_digest_golden(got, "room_grab_w200_s90_ref", ins, exact=EXACT, rtol=1e-4, atol=1e-5)

@@ -8,7 +8,7 @@ import pytest
 
 from oracle import runner
 from sims import SIMS
-from trace_utils import assert_traces_equal, load_golden, make_inputs, rollout_gpu
+from trace_utils import assert_matches_digest_golden, assert_traces_equal, load_golden, make_inputs, rollout_gpu
 
 CFG = {"episode_len": 30, "seed": 8}
 
@@ -38,11 +38,10 @@ def test_gpu_matches_golden():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not runner.available("room_tgs"), reason="oracle/_ref not built")
 def test_gpu_matches_live_reference():
+    # the reference CPU backend's trace is stored as a digest golden (tests/golden/make_golden.py)
     W, steps = 120, 50
     cfg = {"episode_len": 25, "seed": 300}
     ins = make_inputs("room_tgs", W, steps, seed=6)
-    ref, _ = runner.run_reference(SIMS["room_tgs"], W, steps, ins, cfg, workers=4)
     got, _ = rollout_gpu("room_tgs", W, steps, ins, cfg)
-    assert_traces_equal(got, ref)
+    assert_matches_digest_golden(got, "room_tgs_w120_s50_ref", ins)

@@ -2,6 +2,7 @@
 through the C ABI, golden fixture I/O."""
 from __future__ import annotations
 
+import hashlib
 import os
 from typing import Dict
 
@@ -131,3 +132,104 @@ def assert_traces_equal(got, want, exact=True, rtol=1e-4, atol=1e-6):
 
 def golden_path(name: str) -> str:
     return os.path.join(GOLDEN_DIR, name + ".npz")
+
+
+# ---- digest goldens: reference traces too large to store whole ---------------------------
+# Each column is kept as the SHA-256 of its whole trace (a bit-exact comparison), each frame
+# as a short digest of all columns (where a trace starts to differ), and a few seeded values
+# of every tenth frame of the float columns (the 1e-4 comparison of MADRONA_B200_FAST_MATH=1).
+
+SAMPLE_VALUES = 4
+SAMPLE_EVERY = 10
+
+
+def _frames(v):
+    return [np.ascontiguousarray(f) for f in v]
+
+
+def _trace_sha(frames) -> np.ndarray:
+    h = hashlib.sha256()
+    for f in frames:
+        h.update(np.int64(f.shape[0]).tobytes())
+        h.update(f.tobytes())
+    return np.frombuffer(h.digest(), dtype=np.uint8)
+
+
+def _frame_shas(traces, steps) -> np.ndarray:
+    out = np.zeros((steps + 1, 8), dtype=np.uint8)
+    for t in range(steps + 1):
+        out[t] = _trace_sha([traces[k][t] for k in sorted(traces)])[:8]
+    return out
+
+
+def _sample(frames, seed):
+    """SAMPLE_VALUES seeded values of every SAMPLE_EVERY-th frame (dynamic tables: the first ones)."""
+    size = min(f.size for f in frames)
+    idx = np.random.default_rng(seed).choice(size, size=min(SAMPLE_VALUES, size), replace=False)
+    return np.stack([f.reshape(-1)[idx] for f in frames[::SAMPLE_EVERY]]) if size else None
+
+
+def inputs_digest(inputs) -> np.ndarray:
+    h = hashlib.sha256()
+    for k in sorted(inputs or {}):
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(inputs[k]).tobytes())
+    return np.frombuffer(h.digest(), dtype=np.uint8)
+
+
+def save_digest_golden(name, inputs, outs, W, steps):
+    traces = {k: _frames(v) for k, v in outs.items()}
+    payload = {"meta": np.array([W, steps], dtype=np.int64), "in_sha": inputs_digest(inputs),
+               "frame_sha": _frame_shas(traces, steps)}
+    for i, (k, frames) in enumerate(sorted(traces.items())):
+        payload["sha_" + k] = _trace_sha(frames)
+        payload["dtype_" + k] = np.array(frames[0].dtype.str)
+        smp = _sample(frames, i) if np.issubdtype(frames[0].dtype, np.floating) else None
+        if smp is not None:
+            payload["smp_" + k] = smp
+    np.savez_compressed(golden_path(name), **payload)
+
+
+def assert_matches_digest_golden(got, name, inputs, exact=True, rtol=1e-4, atol=1e-6):
+    """`got` (a trace as rollout_gpu returns it) against the digest golden `name`."""
+    z = np.load(golden_path(name))
+    W, steps = (int(v) for v in z["meta"])
+    assert np.array_equal(inputs_digest(inputs), z["in_sha"]), \
+        f"{name}: the inputs differ from the ones the golden trace was made from"
+    keys = sorted(f[4:] for f in z.files if f.startswith("sha_"))
+    traces = {}
+    for i, k in enumerate(keys):
+        assert len(got[k]) == steps + 1, (k, len(got[k]))
+        traces[k] = [np.asarray(f, dtype=np.dtype(str(z["dtype_" + k]))) for f in _frames(got[k])]
+        assert all(f.shape[0] == W for f in traces[k]) or isinstance(got[k], list), k
+    differ = [k for k in keys if not np.array_equal(_trace_sha(traces[k]), z["sha_" + k])]
+    if exact or not differ:
+        if differ:
+            t = int(np.argmax((_frame_shas(traces, steps) != z["frame_sha"]).any(axis=1)))
+            raise AssertionError(f"{name}: columns {differ} differ from the reference, first in frame {t}")
+        return
+    for i, k in enumerate(keys):
+        floating = "smp_" + k in z.files
+        assert floating or k not in differ, f"{k} differs from the reference"
+        if floating:
+            np.testing.assert_allclose(_sample(traces[k], i), z["smp_" + k], rtol=rtol, atol=atol, err_msg=k)
+
+
+# ---- known-answer probes (oracle/*_probe.cpp) ----------------------------------------------
+
+def reference_probe_output(probe: str) -> str:
+    """What the probe printed built against the reference (tests/golden/<probe>.txt.gz)."""
+    import gzip
+    with gzip.open(os.path.join(GOLDEN_DIR, probe + ".txt.gz"), "rt") as f:
+        return f.read()
+
+
+def build_engine_probe(target: str, out_dir) -> str:
+    """Builds oracle/Makefile's `target` (a probe compiled against the engine's own headers
+    only) into out_dir, runs it and returns what it printed."""
+    import subprocess
+    oracle = os.path.join(os.path.dirname(GOLDEN_DIR), os.pardir, "oracle")
+    exe = os.path.join(str(out_dir), target)
+    subprocess.run(["make", "-s", "-C", oracle, "OUT=" + str(out_dir), exe], check=True,
+                   capture_output=True, text=True)
+    return subprocess.run([exe], capture_output=True, text=True, check=True).stdout
