@@ -33,7 +33,7 @@ void setError(const std::string &msg)
         return false; \
     } } while (0)
 
-static bool devAlloc(Executor *ex, void **ptr, size_t bytes, bool zero = true)
+bool devAlloc(Executor *ex, void **ptr, size_t bytes, bool zero)
 {
     if (bytes == 0) bytes = 16;
     MB2_CUDA(cudaMalloc(ptr, bytes));
@@ -91,7 +91,7 @@ static bool launch1(Executor *ex, cudaKernel_t k, unsigned grid, unsigned block)
     return true;
 }
 
-static uint64_t envU64(const char *name, uint64_t dflt)
+uint64_t envU64(const char *name, uint64_t dflt)
 {
     const char *v = getenv(name);
     if (!v || !*v) return dflt;
@@ -247,7 +247,6 @@ bool growTable(Executor *ex, uint32_t a, int64_t new_cap, std::string *err)
     t.capacity = (int32_t)new_cap;
     cudaMemcpy(&ex->dState->tables[a].capacity, &t.capacity, sizeof(int32_t), cudaMemcpyHostToDevice);
     cudaMemcpy(&ex->dState->entityCapacity, &S.entityCapacity, sizeof(int32_t), cudaMemcpyHostToDevice);
-    ex->growthEvents++;
     if (getenv("MADRONA_B200_VERBOSE")) {
         fprintf(stderr, "[madrona_b200] archetype %u grown to %ld rows\n", a, (long)new_cap);
     }
@@ -350,7 +349,6 @@ static bool createExecutor(Executor *ex, const mb2_state_config *sc,
     // torch's `actions.copy_(...)` -- is ordered before the step graph
     MB2_CUDA(cudaStreamCreate(&ex->stream));
     ex->rowsPerWorldHint = envU64("MADRONA_B200_ROWS_PER_WORLD", 128);
-    g_pdl = envU64("MADRONA_B200_PDL", 0) != 0;
     ex->tableGrowth = envU64("MADRONA_B200_TABLE_GROWTH", 1) != 0;
 
     // ---- JIT the simulator
@@ -383,9 +381,7 @@ static bool createExecutor(Executor *ex, const mb2_state_config *sc,
 
     // ---- engine state block
     ex->hState = (EngineState *)calloc(1, sizeof(EngineState));
-    MB2_CUDA(cudaMalloc((void **)&ex->dState, sizeof(EngineState)));
-    ex->allocations.push_back(ex->dState);
-    MB2_CUDA(cudaMemset(ex->dState, 0, sizeof(EngineState)));
+    if (!devAlloc(ex, (void **)&ex->dState, sizeof(EngineState))) return false;
     MB2_CUDA(cudaMallocHost((void **)&ex->hStatus, sizeof(uint32_t) * kStatusWords));
     memset(ex->hStatus, 0, sizeof(uint32_t) * kStatusWords);
 
@@ -560,16 +556,7 @@ static bool enqueueNode(Executor *ex, uint32_t node_idx, cudaStream_t s)
         unsigned grid = (unsigned)std::max<uint64_t>(1, std::min(blocks, max_blocks));
         const NodeRecord *drec = &ex->dState->nodes[node_idx];
         void *args[1] = { (void *)&drec };
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(grid);
-        cfg.blockDim = dim3(256);
-        cfg.stream = s;
-        cudaLaunchAttribute attr;
-        attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr.val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
-        cfg.attrs = &attr;
-        cfg.numAttrs = 1;
-        MB2_CUDA(cudaLaunchKernelExC(&cfg, (const void *)ex->nodeKernels[r.kernelID], args));
+        MB2_CUDA(cudaLaunchKernel((const void *)ex->nodeKernels[r.kernelID], dim3(grid), dim3(256), args, 0, s));
         return true;
     }
     case NodeSortArchetype:
@@ -618,13 +605,12 @@ static bool enqueueNode(Executor *ex, uint32_t node_idx, cudaStream_t s)
     }
 }
 
-static LaunchGraph *buildGraph(Executor *ex, const uint32_t *ids, uint32_t n, const char *name)
+static LaunchGraph *buildGraph(Executor *ex, const uint32_t *ids, uint32_t n)
 {
     EngineState &S = *ex->hState;
     cudaSetDevice(ex->gpu);
     LaunchGraph *g = new LaunchGraph();
     g->owner = ex;
-    g->name = name ? name : "";
 
     physicsBeforeGraphCapture(ex);
 
@@ -1034,11 +1020,12 @@ mb2_executor *mb2_executor_create(const mb2_state_config *state_cfg,
 
 void mb2_executor_destroy(mb2_executor *exec) { destroyExecutor((Executor *)exec); }
 
+// stat_name is part of the reference's signature; this executor keeps no per-graph statistics
 mb2_launch_graph *mb2_build_launch_graph(mb2_executor *exec, const uint32_t *taskgraph_ids,
-                                         uint32_t num_taskgraphs, const char *stat_name)
+                                         uint32_t num_taskgraphs, const char * /*stat_name*/)
 {
     g_last_error.clear();
-    return (mb2_launch_graph *)buildGraph((Executor *)exec, taskgraph_ids, num_taskgraphs, stat_name);
+    return (mb2_launch_graph *)buildGraph((Executor *)exec, taskgraph_ids, num_taskgraphs);
 }
 
 mb2_launch_graph *mb2_build_launch_graph_all(mb2_executor *exec)

@@ -49,7 +49,6 @@ struct Executor {
     std::vector<VMRange> columnRanges[kMaxArchetypes];         // [archetype][column]; empty: fixed table
     std::vector<VMRange> twinRanges[kMaxArchetypes];
     VMRange entityRange;
-    int64_t growthEvents = 0;
 };
 
 // status block published by the last kernel of every launch graph (pinned host memory)
@@ -61,40 +60,16 @@ struct LaunchGraph {
     cudaGraphExec_t exec = nullptr;
     int64_t numKernels = 0;
     int64_t numBranches = 1;   // capture streams used (parallel branches of independent nodes)
-    std::string name;
 };
 
 void setError(const std::string &msg);
 
-// Programmatic dependent launch (MADRONA_B200_PDL=1, default OFF): every engine
-// kernel starts with mb2::pdlSync() -- "let my dependents be scheduled now, then
-// wait for my prerequisites to have completed" -- and can be launched with the
-// programmatic stream-serialization attribute, so that the ~50 kernel -> kernel
-// edges of the captured step graph do not each pay a drain + launch latency.
-// Measured on B200 (A/B in one run): room 1.044 -> 1.164 ms/step, arena 1.556 ->
-// 1.936 with it ON: the step's kernels are multi-wave (4096 blocks over ~1200
-// resident slots) and the parked blocks of the next kernel take slots from the
-// current kernel's later waves.  Kept behind the switch; with it off pdlSync()
-// is two no-op instructions.
-extern bool g_pdl;
+// unsigned environment variable, `dflt` when unset or empty
+uint64_t envU64(const char *name, uint64_t dflt);
 
-#ifdef __CUDACC__
-template <typename... KArgs, typename... Args>
-inline void launchK(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args)
-{
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr.val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-#endif
+// cudaMalloc'd block owned by the executor (freed with it), zeroed on ex->stream unless
+// `zero` is false; a zero-byte request gets 16 bytes.  On failure: setError and false.
+bool devAlloc(Executor *ex, void **ptr, size_t bytes, bool zero = true);
 
 // ---- ahead-of-time engine kernels (kernels_core.cu / kernels_sort.cu) -----
 void launchClearTmp(Executor *ex, uint32_t archetype, cudaStream_t s);

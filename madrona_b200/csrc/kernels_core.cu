@@ -5,13 +5,10 @@
 
 namespace mb2 {
 
-bool g_pdl = false;
-
 // ClearTmpNode: drop every row of a temporary archetype (numRows.exchange(0)
 // in the reference) and zero its per-world counts.
 __global__ void clearTmpKernel(EngineState *S, uint32_t archetype)
 {
-    pdlSync();
     TableDesc &t = S->tables[archetype];
     const int32_t W = (int32_t)S->numWorlds;
     for (int32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < W; w += gridDim.x * blockDim.x) {
@@ -27,14 +24,12 @@ __global__ void clearTmpKernel(EngineState *S, uint32_t archetype)
 
 __global__ void resetTmpAllocKernel(EngineState *S)
 {
-    pdlSync();
     S->tmpOffset = 0;
 }
 
 // Last node of every launch graph: publish error flags to pinned host memory.
 __global__ void statusCopyKernel(EngineState *S, uint32_t *host_status)
 {
-    pdlSync();
     host_status[0] = S->errorFlags;
     host_status[1] = S->errorArchetype;
     // peak row count of every table during this graph (the host grows tables between steps)
@@ -51,7 +46,6 @@ __global__ void statusCopyKernel(EngineState *S, uint32_t *host_status)
 // entity IDs follow the CPU backend's init cache: order * W + world.
 __global__ void fillSingletonsKernel(EngineState *S)
 {
-    pdlSync();
     const int32_t W = (int32_t)S->numWorlds;
     for (uint32_t a = 0; a < S->numArchetypes; a++) {
         const ArchetypeInfo &info = S->archetypes[a];
@@ -74,23 +68,23 @@ __global__ void fillSingletonsKernel(EngineState *S)
 void launchClearTmp(Executor *ex, uint32_t archetype, cudaStream_t s)
 {
     int grid = (int)std::min<uint32_t>((ex->hState->numWorlds + 255) / 256, (uint32_t)ex->numSMs * 2);
-    launchK(clearTmpKernel, dim3(std::max(grid, 1)), dim3(256), 0, s, ex->dState, archetype);
+    clearTmpKernel<<<std::max(grid, 1), 256, 0, s>>>(ex->dState, archetype);
 }
 
 void launchResetTmpAlloc(Executor *ex, cudaStream_t s)
 {
-    launchK(resetTmpAllocKernel, dim3(1), dim3(1), 0, s, ex->dState);
+    resetTmpAllocKernel<<<1, 1, 0, s>>>(ex->dState);
 }
 
 void launchStatusCopy(Executor *ex, cudaStream_t s)
 {
-    launchK(statusCopyKernel, dim3(1), dim3(32), 0, s, ex->dState, ex->hStatus);
+    statusCopyKernel<<<1, 32, 0, s>>>(ex->dState, ex->hStatus);
 }
 
 void launchFillSingletons(Executor *ex, cudaStream_t s)
 {
     int grid = (int)std::min<uint32_t>((ex->hState->numWorlds + 255) / 256, (uint32_t)ex->numSMs * 2);
-    launchK(fillSingletonsKernel, dim3(std::max(grid, 1)), dim3(256), 0, s, ex->dState);
+    fillSingletonsKernel<<<std::max(grid, 1), 256, 0, s>>>(ex->dState);
 }
 
 }

@@ -1783,7 +1783,6 @@ template <bool SPHERE_HULL>
 __global__ void __launch_bounds__(kNarrowSimpleThreads, MB2_NS_MINB)
 physNarrowSimpleKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     const PhysicsState &P = *S.physics;
     fillColCache(S, P);
@@ -1847,7 +1846,6 @@ constexpr int kNarrowHullThreads = 64;
 __global__ void __launch_bounds__(kNarrowHullThreads, MB2_NH_MINB)
 physNarrowHullKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     const PhysicsState &P = *S.physics;
     fillColCache(S, P);
@@ -2411,11 +2409,13 @@ enum PhysPhase : u32 {
 #ifndef MB2_BODY_MINB
 #define MB2_BODY_MINB 1
 #endif
+#ifndef MB2_BODY_BLOCKS_PER_SM
+#define MB2_BODY_BLOCKS_PER_SM 4
+#endif
 template <u32 OP>
 __global__ void __launch_bounds__(256, MB2_BODY_MINB)
 physBodyKernel(EngineState *Sp)
 {
-    pdlSync();
     const EngineState &S = *Sp;
     const PhysicsState &P = *S.physics;
     if (blockIdx.y >= P.numBodyArchetypes) return;
@@ -2444,7 +2444,6 @@ physBodyKernel(EngineState *Sp)
 __global__ void __launch_bounds__(128)
 physRebuildKernel(EngineState *Sp)
 {
-    pdlSync();
     const EngineState &S = *Sp;
     const i32 w = blockIdx.x * blockDim.x + threadIdx.x;
     if (w >= (i32)S.numWorlds) return;
@@ -2472,16 +2471,10 @@ __device__ __forceinline__ void forEachWorldBody(const EngineState &S, const Phy
 // into one launch -- integrate -> narrowphase, position solve -> velocity update
 // -> velocity solve -- was measured: no gain, and the bigger kernels miss the
 // 32 KB instruction cache more; see DESIGN.md 3.2.)
-#ifndef MB2_NARROW_MINB
-#define MB2_NARROW_MINB 8
-#endif
-constexpr int physMinBlocks(u32) { return 8; }
-
 template <u32 OP>
-__global__ void __launch_bounds__(32 * kPhysWarps, physMinBlocks(OP))
+__global__ void __launch_bounds__(32 * kPhysWarps, 8)
 physWorldKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     const PhysicsState &P = *S.physics;
     fillColCache(S, P);
@@ -2525,20 +2518,12 @@ bool physicsHostCreate(Executor *ex, std::string *err)
     PhysicsHost *ph = new PhysicsHost();
     ex->physics = ph;
     memset(&ph->hPhys, 0, sizeof(PhysicsState));
-    if (cudaMalloc((void **)&ph->dPhys, sizeof(PhysicsState)) != cudaSuccess) {
+    if (!devAlloc(ex, (void **)&ph->dPhys, sizeof(PhysicsState))) {
         *err = "physics state allocation failed";
         return false;
     }
-    ex->allocations.push_back(ph->dPhys);
-    cudaMemset(ph->dPhys, 0, sizeof(PhysicsState));
     ex->hState->physics = ph->dPhys;
     return true;
-}
-
-static uint64_t envU64p(const char *name, uint64_t dflt)
-{
-    const char *v = getenv(name);
-    return (v && *v) ? strtoull(v, nullptr, 10) : dflt;
 }
 
 bool physicsHostAfterRegistry(Executor *ex, const mb2_render_config *, std::string *err)
@@ -2576,24 +2561,18 @@ bool physicsHostAfterRegistry(Executor *ex, const mb2_render_config *, std::stri
     }
     P.jointCol = S.columnLookup[P.jointArchetype][P.cidJointConstraint];
 
-    P.maxCandidatesPerWorld = (i32)envU64p("MADRONA_B200_MAX_CANDIDATES_PER_WORLD", 256);
-    P.maxContactsPerWorld = (i32)envU64p("MADRONA_B200_MAX_CONTACTS_PER_WORLD", 128);
+    P.maxCandidatesPerWorld = (i32)envU64("MADRONA_B200_MAX_CANDIDATES_PER_WORLD", 256);
+    P.maxContactsPerWorld = (i32)envU64("MADRONA_B200_MAX_CONTACTS_PER_WORLD", 128);
     const size_t W = S.numWorlds;
-    auto alloc = [&](void **p, size_t bytes) {
-        if (cudaMalloc(p, bytes) != cudaSuccess) return false;
-        ex->allocations.push_back(*p);
-        cudaMemset(*p, 0, bytes);
-        return true;
-    };
-    if (!alloc((void **)&P.candidates, sizeof(Candidate) * W * P.maxCandidatesPerWorld) ||
-        !alloc((void **)&P.candCounts, sizeof(i32) * W) ||
-        !alloc((void **)&P.contacts, sizeof(Contact) * W * P.maxCandidatesPerWorld) ||
-        !alloc((void **)&P.candHit, sizeof(i32) * W * P.maxCandidatesPerWorld) ||
-        !alloc((void **)&P.contactOrder, sizeof(i32) * W * P.maxContactsPerWorld) ||
-        !alloc((void **)&P.hullQueue, sizeof(HullQueueEntry) * W * P.maxCandidatesPerWorld) ||
-        !alloc((void **)&P.hullQueueCount, sizeof(i32) * 4) ||
-        !alloc((void **)&P.contactCounts, sizeof(i32) * W) ||
-        !alloc((void **)&P.contactMaxLevel, sizeof(i32) * W)) {
+    if (!devAlloc(ex, (void **)&P.candidates, sizeof(Candidate) * W * P.maxCandidatesPerWorld) ||
+        !devAlloc(ex, (void **)&P.candCounts, sizeof(i32) * W) ||
+        !devAlloc(ex, (void **)&P.contacts, sizeof(Contact) * W * P.maxCandidatesPerWorld) ||
+        !devAlloc(ex, (void **)&P.candHit, sizeof(i32) * W * P.maxCandidatesPerWorld) ||
+        !devAlloc(ex, (void **)&P.contactOrder, sizeof(i32) * W * P.maxContactsPerWorld) ||
+        !devAlloc(ex, (void **)&P.hullQueue, sizeof(HullQueueEntry) * W * P.maxCandidatesPerWorld) ||
+        !devAlloc(ex, (void **)&P.hullQueueCount, sizeof(i32) * 4) ||
+        !devAlloc(ex, (void **)&P.contactCounts, sizeof(i32) * W) ||
+        !devAlloc(ex, (void **)&P.contactMaxLevel, sizeof(i32) * W)) {
         *err = "physics buffers allocation failed";
         return false;
     }
@@ -2623,11 +2602,7 @@ static dim3 bodyGrid(Executor *ex)
     for (uint32_t i = 0; i < P.numBodyArchetypes; i++) {
         max_cap = std::max(max_cap, ex->hState->tables[P.bodies[i].archetype].capacity);
     }
-    static const int per_sm = [] {
-        const char *v = getenv("MADRONA_B200_BODY_BLOCKS_PER_SM");
-        return (v && *v) ? std::max(1, atoi(v)) : 4;
-    }();
-    int blocks = std::min((max_cap + 255) / 256, ex->numSMs * per_sm);
+    int blocks = std::min((max_cap + 255) / 256, ex->numSMs * MB2_BODY_BLOCKS_PER_SM);
     return dim3((unsigned)std::max(blocks, 1), std::max(P.numBodyArchetypes, 1u));
 }
 
@@ -2653,40 +2628,40 @@ bool physicsEnqueueNodes(Executor *ex, const NodeRecord *recs, uint32_t count, c
             // tag 0 (post-integration) never rebuilds in the reference either; a
             // pending rebuild request then simply waits for the next tag-1 node,
             // and the un-refitted leaves are refitted by that rebuild
-            launchK(physBodyKernel<PhaseUpdateLeaves>, dim3(bgrid), dim3(256), 0, s, d);
-            if (rec.userTag == 1) launchK(physRebuildKernel, dim3((W + 127) / 128), dim3(128), 0, s, d);
+            physBodyKernel<PhaseUpdateLeaves><<<bgrid, 256, 0, s>>>(d);
+            if (rec.userTag == 1) physRebuildKernel<<<(W + 127) / 128, 128, 0, s>>>(d);
             break;
         case NodePhysFindCandidates:
             // joints are iterated per world by the solver: keep their table in
             // world order (the reference sorts Joint here too, xpbd.cpp:1092-1096)
             launchSortArchetype(ex, ph->hPhys.jointArchetype, 1, s);
-            launchK(physWorldKernel<PhaseFindCandidates>, dim3(wgrid), dim3(wblock), 0, s, d);
+            physWorldKernel<PhaseFindCandidates><<<wgrid, wblock, 0, s>>>(d);
             break;
         case NodePhysSubstepBegin:
-            launchK(physBodyKernel<PhaseIntegrate>, dim3(bgrid), dim3(256), 0, s, d);
+            physBodyKernel<PhaseIntegrate><<<bgrid, 256, 0, s>>>(d);
             break;
         case NodePhysNarrowphase:
             {
                 const unsigned sgrid_n = (W + kNarrowWorldsPerBlock - 1) / kNarrowWorldsPerBlock;
-                if (ph->spheres) launchK(physNarrowSimpleKernel<true>, dim3(sgrid_n), dim3(kNarrowSimpleThreads), 0, s, d);
-                else launchK(physNarrowSimpleKernel<false>, dim3(sgrid_n), dim3(kNarrowSimpleThreads), 0, s, d);
-                launchK(physNarrowHullKernel, dim3((unsigned)ex->numSMs * (unsigned)MB2_NH_MINB), dim3(kNarrowHullThreads), 0, s, d);
+                if (ph->spheres) physNarrowSimpleKernel<true><<<sgrid_n, kNarrowSimpleThreads, 0, s>>>(d);
+                else physNarrowSimpleKernel<false><<<sgrid_n, kNarrowSimpleThreads, 0, s>>>(d);
+                physNarrowHullKernel<<<(unsigned)ex->numSMs * (unsigned)MB2_NH_MINB, kNarrowHullThreads, 0, s>>>(d);
             }
             break;
         case NodePhysSolvePositions:
-            launchK(physWorldKernel<PhaseSolvePositions>, dim3(sgrid), dim3(wblock), 0, s, d);
+            physWorldKernel<PhaseSolvePositions><<<sgrid, wblock, 0, s>>>(d);
             break;
         case NodePhysTGSVelocities:
-            launchK(physBodyKernel<PhaseTGSVelocities>, dim3(bgrid), dim3(256), 0, s, d);
+            physBodyKernel<PhaseTGSVelocities><<<bgrid, 256, 0, s>>>(d);
             break;
         case NodePhysTGSPositions:
-            launchK(physBodyKernel<PhaseTGSPositions>, dim3(bgrid), dim3(256), 0, s, d);
+            physBodyKernel<PhaseTGSPositions><<<bgrid, 256, 0, s>>>(d);
             break;
         case NodePhysSetVelocities:
-            launchK(physBodyKernel<PhaseSetVelocities>, dim3(bgrid), dim3(256), 0, s, d);
+            physBodyKernel<PhaseSetVelocities><<<bgrid, 256, 0, s>>>(d);
             break;
         case NodePhysSolveVelocities:
-            launchK(physWorldKernel<PhaseSolveVelocities>, dim3(sgrid), dim3(wblock), 0, s, d);
+            physWorldKernel<PhaseSolveVelocities><<<sgrid, wblock, 0, s>>>(d);
             break;
         default:
             *err = "unknown physics node kind " + std::to_string(rec.kind);

@@ -71,7 +71,6 @@ struct RenderCameraComp {     // == madrona::render::RenderCamera
 __global__ void __launch_bounds__(128)
 renderGatherInstancesKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     RenderState &R = *S.render;
     const int lane = threadIdx.x & 31;
@@ -141,7 +140,6 @@ __global__ void __launch_bounds__(256)
 renderLightUpdateKernel(EngineState *Sp, u32 archetype, i32 carrier_col, i32 pos_col, i32 dir_col, i32 type_col,
                         i32 shadow_col, i32 cutoff_col, i32 intensity_col, i32 active_col)
 {
-    pdlSync();
     EngineState &S = *Sp;
     const RenderState &R = *S.render;
     const TableDesc &t = S.tables[archetype];
@@ -170,7 +168,6 @@ renderLightUpdateKernel(EngineState *Sp, u32 archetype, i32 carrier_col, i32 pos
 __global__ void __launch_bounds__(256)
 renderGatherLightsKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     RenderState &R = *S.render;
     const TableDesc &t = S.tables[R.lightArchetype];
@@ -204,7 +201,6 @@ renderGatherLightsKernel(EngineState *Sp)
 __global__ void __launch_bounds__(256)
 renderGatherViewsKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     RenderState &R = *S.render;
     if (blockIdx.y >= R.numViewArchetypes) return;
@@ -294,7 +290,6 @@ __device__ __forceinline__ int commonPrefix(const unsigned long long *keys, int 
 __global__ void __launch_bounds__(32)
 renderBuildTLASKernel(EngineState *Sp)
 {
-    pdlSync();
     extern __shared__ __align__(16) unsigned char tlas_smem[];
     EngineState &S = *Sp;
     RenderState &R = *S.render;
@@ -848,7 +843,6 @@ template <bool FLAT>
 __global__ void __launch_bounds__(256, MB2_RAYCAST_MINB)
 renderRaycastKernel(EngineState *Sp)
 {
-    pdlSync();
     EngineState &S = *Sp;
     const RenderState &R = *S.render;
     const TableDesc &out_tbl = S.tables[R.outputArchetype];
@@ -1109,11 +1103,10 @@ bool renderHostCreate(Executor *ex, const mb2_render_config *rc, std::string *er
     RenderHost *rh = new RenderHost();
     ex->render = rh;
     memset(&rh->hRender, 0, sizeof(RenderState));
-    if (cudaMalloc((void **)&rh->dRender, sizeof(RenderState)) != cudaSuccess) {
+    if (!devAlloc(ex, (void **)&rh->dRender, sizeof(RenderState), false)) {
         *err = "render state allocation failed";
         return false;
     }
-    ex->allocations.push_back(rh->dRender);
     RenderState &R = rh->hRender;
     if (rc && rc->render_resolution > 0) {
         if (!rc->geo_bvh_data.mesh_bvhs || rc->geo_bvh_data.num_bvhs == 0) {
@@ -1226,22 +1219,16 @@ bool renderHostAfterRegistry(Executor *ex, std::string *err)
         }
     }
 
-    auto alloc = [&](void **p, size_t bytes) {
-        if (cudaMalloc(p, bytes) != cudaSuccess) return false;
-        ex->allocations.push_back(*p);
-        cudaMemset(*p, 0, bytes);
-        return true;
-    };
     const size_t W = S.numWorlds;
-    if (!alloc((void **)&R.instances, sizeof(RenderInstance) * W * R.maxInstancesPerWorld) ||
-        !alloc((void **)&R.instanceCounts, sizeof(i32) * W) ||
-        !alloc((void **)&R.tlasNodes, sizeof(QBVHNode) * W * R.maxInstancesPerWorld) ||
-        !alloc((void **)&R.tlasNodeCounts, sizeof(i32) * W) ||
-        !alloc((void **)&R.lights, sizeof(RenderLight) * W * kMaxLightsPerWorld) ||
-        !alloc((void **)&R.lightCounts, sizeof(i32) * W) ||
-        (R.debugHits && !alloc((void **)&R.hitIDs, sizeof(i32) * 2 * (size_t)R.maxViews * R.resolution *
-                                                       R.resolution)) ||
-        !alloc((void **)&R.views, sizeof(RenderView) * (size_t)R.maxViews)) {
+    if (!devAlloc(ex, (void **)&R.instances, sizeof(RenderInstance) * W * R.maxInstancesPerWorld) ||
+        !devAlloc(ex, (void **)&R.instanceCounts, sizeof(i32) * W) ||
+        !devAlloc(ex, (void **)&R.tlasNodes, sizeof(QBVHNode) * W * R.maxInstancesPerWorld) ||
+        !devAlloc(ex, (void **)&R.tlasNodeCounts, sizeof(i32) * W) ||
+        !devAlloc(ex, (void **)&R.lights, sizeof(RenderLight) * W * kMaxLightsPerWorld) ||
+        !devAlloc(ex, (void **)&R.lightCounts, sizeof(i32) * W) ||
+        (R.debugHits && !devAlloc(ex, (void **)&R.hitIDs, sizeof(i32) * 2 * (size_t)R.maxViews * R.resolution *
+                                                              R.resolution)) ||
+        !devAlloc(ex, (void **)&R.views, sizeof(RenderView) * (size_t)R.maxViews)) {
         *err = "render buffers allocation failed";
         return false;
     }
@@ -1257,7 +1244,6 @@ void renderHostDestroy(Executor *ex)
 
 __global__ void renderResetCountsKernel(EngineState *Sp)
 {
-    pdlSync();
     Sp->render->totalNumInstances = 0;
 }
 
@@ -1268,25 +1254,25 @@ bool renderEnqueuePrepare(Executor *ex, cudaStream_t s, std::string *err)
     (void)err;
     const RenderState &R = rh->hRender;
     const unsigned W = ex->hState->numWorlds;
-    launchK(renderResetCountsKernel, dim3(1), dim3(1), 0, s, ex->dState);
-    launchK(renderGatherInstancesKernel, dim3((W * 32 + 127) / 128), dim3(128), 0, s, ex->dState);
+    renderResetCountsKernel<<<1, 1, 0, s>>>(ex->dState);
+    renderGatherInstancesKernel<<<(W * 32 + 127) / 128, 128, 0, s>>>(ex->dState);
     // lights: carriers refresh their light entities, the light table is brought into
     // world order (no-op when clean), then listed per world
     for (const LightCarrierArchetype &lc : lightCarriers(ex)) {
         const int cap = ex->hState->tables[lc.archetype].capacity;
-        launchK(renderLightUpdateKernel, dim3((unsigned)std::max(1, std::min((cap + 255) / 256, ex->numSMs * 2))),
-                dim3(256), 0, s, ex->dState, lc.archetype, lc.carrierCol, lc.posCol, lc.dirCol, lc.typeCol,
-                lc.shadowCol, lc.cutoffCol, lc.intensityCol, lc.activeCol);
+        renderLightUpdateKernel<<<(unsigned)std::max(1, std::min((cap + 255) / 256, ex->numSMs * 2)), 256, 0, s>>>(
+            ex->dState, lc.archetype, lc.carrierCol, lc.posCol, lc.dirCol, lc.typeCol,
+            lc.shadowCol, lc.cutoffCol, lc.intensityCol, lc.activeCol);
     }
     launchSortArchetype(ex, R.lightArchetype, 1, s);
-    launchK(renderGatherLightsKernel, dim3((W + 255) / 256), dim3(256), 0, s, ex->dState);
+    renderGatherLightsKernel<<<(W + 255) / 256, 256, 0, s>>>(ex->dState);
     int max_cap = 256;
     for (u32 i = 0; i < R.numViewArchetypes; i++) {
         max_cap = std::max(max_cap, ex->hState->tables[R.viewers[i].archetype].capacity);
     }
     dim3 grid((unsigned)std::min((max_cap + 255) / 256, ex->numSMs * 4), std::max(R.numViewArchetypes, 1u));
-    launchK(renderGatherViewsKernel, dim3(grid), dim3(256), 0, s, ex->dState);
-    launchK(renderBuildTLASKernel, dim3(W), dim3(32), rh->tlasSmem, s, ex->dState);
+    renderGatherViewsKernel<<<grid, 256, 0, s>>>(ex->dState);
+    renderBuildTLASKernel<<<W, 32, rh->tlasSmem, s>>>(ex->dState);
     return true;
 }
 
@@ -1322,7 +1308,6 @@ LaunchGraph *physicsBuildRenderGraph(Executor *ex, std::string *err)
     const RenderState &R = rh->hRender;
     LaunchGraph *g = new LaunchGraph();
     g->owner = ex;
-    g->name = "render";
     cudaSetDevice(ex->gpu);
     if (cudaStreamBeginCapture(ex->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
         *err = "cudaStreamBeginCapture failed";
@@ -1333,8 +1318,8 @@ LaunchGraph *physicsBuildRenderGraph(Executor *ex, std::string *err)
     // the live view count: one block per capacity row cost 76 us of empty-block scheduling at
     // 1024 worlds); 8 rounds of resident blocks keep the tail short
     const unsigned view_blocks = (unsigned)std::max(1, std::min(R.maxViews, ex->numSMs * MB2_RAYCAST_MINB * 8));
-    launchK(renderRaycastKernel<true>, dim3(1, view_blocks), dim3(256), 0, ex->stream, ex->dState);
-    launchK(renderRaycastKernel<false>, dim3(1, view_blocks), dim3(256), 0, ex->stream, ex->dState);
+    renderRaycastKernel<true><<<dim3(1, view_blocks), 256, 0, ex->stream>>>(ex->dState);
+    renderRaycastKernel<false><<<dim3(1, view_blocks), 256, 0, ex->stream>>>(ex->dState);
     launchStatusCopy(ex, ex->stream);
     cudaError_t e = cudaStreamEndCapture(ex->stream, &g->graph);
     if (e != cudaSuccess || cudaGraphInstantiate(&g->exec, g->graph, 0) != cudaSuccess) {

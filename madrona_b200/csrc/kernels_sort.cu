@@ -21,12 +21,9 @@
 //                        pointers are flipped on the device, so no copy-back;
 //                        also entity remap + offsets/counts + scratch reset)
 // => P+2 launches per sort.  Exported columns must keep their address, so
-// they (only) get one extra copy-back launch (or, behind
-// MADRONA_B200_SORT_FUSE_COPYBACK=1, copy-back items inside the rearrange
-// kernel -- measured slower on B200, DESIGN.md 3.1).
+// they (only) get one extra copy-back launch.
 #include "engine.hpp"
 #include <cstdio>
-#include <cstdlib>
 
 namespace mb2 {
 
@@ -46,7 +43,6 @@ struct SortCtrl {
     int32_t didSort;
     int32_t copyBlocksDone;
     int32_t moveTicket;               // rearrange work-item ticket
-    int32_t colDone[kMaxColumns];     // gather chunks finished per column (copy-back items wait on it)
 };
 
 struct SortScratch {
@@ -77,8 +73,6 @@ struct SortParams {
     void **alt;       // this archetype's row of altColumns
     int32_t maxTiles;
     int32_t hasExported;
-    int32_t fuseCopyBack;             // exported columns are copied back inside the rearrange kernel
-    unsigned long long exportedMask;
 };
 
 // ---- TMA (bulk async copy) staging of contiguous tiles: global -> shared memory by the
@@ -143,7 +137,6 @@ __device__ __forceinline__ uint32_t loadKey(const TableDesc &t, int32_t col, int
 __global__ void __launch_bounds__(kSortThreads)
 sortHistogramKernel(SortParams p)
 {
-    pdlSync();
     const TableDesc &t = p.state->tables[p.archetype];
     if (!sortActive(p, t)) return;
     const int32_t n = t.numRows;
@@ -181,11 +174,16 @@ constexpr uint32_t kValueMask = (1u << 30) - 1u;
 #define MB2_SORT_LOOK_WINDOW 8
 #endif
 constexpr int kLookWindow = MB2_SORT_LOOK_WINDOW;
+// ticketed tiles: any grid size is deadlock free; more resident blocks hide the
+// ranking / look-back latency of each tile
+// (B200, 3.1M rows: 2 -> 0.659, 3 -> 0.615, 4 -> 0.598, 6 -> 0.599 ms)
+#ifndef MB2_SWEEP_BLOCKS_PER_SM
+#define MB2_SWEEP_BLOCKS_PER_SM 4
+#endif
 
 __global__ void __launch_bounds__(kSortThreads, 4)
 sortOnesweepKernel(SortParams p, int pass)
 {
-    pdlSync();
     const TableDesc &t = p.state->tables[p.archetype];
     if (!sortActive(p, t)) return;
     const int32_t n = t.numRows;
@@ -421,17 +419,14 @@ sortOnesweepKernel(SortParams p, int pass)
 // in its widest aligned unit (16/8/4/1 bytes) with coalesced stores, four independent
 // gathers in flight per thread.
 //
-// Exported columns must keep their address.  With fuseCopyBack (off by default) their copy-back items
-// (twin -> exported address, 16-byte units) follow the column's gather items in ticket
-// order and wait on the column's chunk counter, so the twin is re-read while it is still
-// in L2 and no extra launch is needed.  Deadlock free for any grid size: a copy-back item
-// waits only for gather items with smaller tickets, which are held by running blocks and
-// never wait themselves.
-//
 // The same kernel re-points entity slots, derives worldOffsets/worldCounts from the sorted
 // keys and wipes the look-back scratch; the last block flips the column pointers and
 // publishes the new row count.
 constexpr int kRearrangeTile = 2048;
+// (B200, sortcheck: 4 -> 0.459, 8 -> 0.458 ms/step, profiles/r2b_ab_table.txt)
+#ifndef MB2_REARRANGE_BLOCKS_PER_SM
+#define MB2_REARRANGE_BLOCKS_PER_SM 8
+#endif
 
 template <typename UnitT>
 __device__ __forceinline__ void gatherTile(const void *src_v, void *dst_v, const int32_t *perm_s,
@@ -469,7 +464,6 @@ __device__ __forceinline__ void gatherTile(const void *src_v, void *dst_v, const
 __global__ void __launch_bounds__(256)
 sortRearrangeKernel(SortParams p)
 {
-    pdlSync();
     TableDesc &t = p.state->tables[p.archetype];
     if (!sortActive(p, t)) return;
     const int32_t n = t.numRows;
@@ -478,7 +472,6 @@ sortRearrangeKernel(SortParams p)
     const int32_t *perm = p.idx[last];
     const uint32_t *sorted_keys = p.keys[last];
     const int32_t num_cols = t.numColumns;
-    const unsigned long long fused_mask = p.fuseCopyBack ? p.exportedMask : 0ull;
 
     __shared__ __align__(128) int32_t perm_s[kRearrangeTile];
     __shared__ __align__(8) unsigned long long perm_bar;
@@ -508,10 +501,9 @@ sortRearrangeKernel(SortParams p)
         }
     }
 
-    // ---- column moves: ticketed (phase, chunk) items; phases = G(col 0) [C(col 0)] G(col 1) ...
+    // ---- column moves: ticketed (column, chunk) items in column-major order
     const int32_t chunks = (new_n + kRearrangeTile - 1) / kRearrangeTile;
-    const int32_t num_phases = num_cols + __popcll(fused_mask & ((num_cols >= 64) ? ~0ull : ((1ull << num_cols) - 1ull)));
-    const int64_t num_items = (int64_t)chunks * num_phases;
+    const int64_t num_items = (int64_t)chunks * num_cols;
     int32_t staged_chunk = -1;      // which slice of the permutation perm_s holds
     while (true) {
         __syncthreads();            // the previous item is done with perm_s / item_s
@@ -519,43 +511,11 @@ sortRearrangeKernel(SortParams p)
         __syncthreads();
         const int64_t item = item_s;
         if (item >= num_items) break;
-        int32_t phase = (int32_t)(item / chunks);
-        const int32_t chunk = (int32_t)(item - (int64_t)phase * chunks);
-        // phase -> (column, gather | copy-back)
-        int32_t col = 0;
-        bool copy_back = false;
-        for (; col < num_cols; col++) {
-            const int32_t span = 1 + (int32_t)((fused_mask >> col) & 1ull);
-            if (phase < span) { copy_back = phase == 1; break; }
-            phase -= span;
-        }
+        const int32_t col = (int32_t)(item / chunks);
+        const int32_t chunk = (int32_t)(item - (int64_t)col * chunks);
         const int32_t row0 = chunk * kRearrangeTile;
         const int32_t rows = min(kRearrangeTile, new_n - row0);
         const uint32_t bytes = t.columnBytes[col];
-
-        if (copy_back) {
-            // every gather chunk of this column has landed in the twin
-            if (threadIdx.x == 0) {
-                volatile int32_t *done = &p.ctrl->colDone[col];
-                while (*done < chunks) { }
-                __threadfence();
-            }
-            __syncthreads();
-            // (columns are 256-byte aligned with 256 bytes of slack: whole 16-byte units;
-            //  row0 * bytes is a multiple of 2048)
-            const uint4 *src = (const uint4 *)((const char *)p.alt[col] + (size_t)row0 * bytes);
-            uint4 *dst = (uint4 *)((char *)t.columns[col] + (size_t)row0 * bytes);
-            const uint32_t units = (uint32_t)(((size_t)rows * bytes + 15) / 16);
-            const uint32_t B = blockDim.x;
-            uint32_t i = threadIdx.x;
-            for (; i + 3 * B < units; i += 4 * B) {
-                const uint4 a = __ldcg(src + i), b = __ldcg(src + i + B);
-                const uint4 c = __ldcg(src + i + 2 * B), d = __ldcg(src + i + 3 * B);
-                dst[i] = a; dst[i + B] = b; dst[i + 2 * B] = c; dst[i + 3 * B] = d;
-            }
-            for (; i < units; i += B) dst[i] = __ldcg(src + i);
-            continue;
-        }
 
         if (staged_chunk != chunk) {
             if (rows == kRearrangeTile) {
@@ -603,12 +563,6 @@ sortRearrangeKernel(SortParams p)
         } else {
             gatherTile<unsigned char>(src, dst, perm_s, row0, rows, bytes);
         }
-        if ((fused_mask >> col) & 1ull) {
-            // publish the chunk to the column's copy-back items
-            __threadfence();
-            __syncthreads();
-            if (threadIdx.x == 0) atomicAdd(&p.ctrl->colDone[col], 1);
-        }
     }
 
     // ---- last block out: flip column buffers, publish the new row count
@@ -624,8 +578,6 @@ sortRearrangeKernel(SortParams p)
     __threadfence();
 
     for (int c = threadIdx.x; c < num_cols; c += blockDim.x) {
-        p.ctrl->colDone[c] = 0;
-        if ((fused_mask >> c) & 1ull) continue;     // already back at its exported address
         void *old_main = t.columns[c];
         t.columns[c] = p.alt[c];
         p.alt[c] = old_main;
@@ -641,7 +593,7 @@ sortRearrangeKernel(SortParams p)
         p.ctrl->numDeleted = 0;
         p.ctrl->blocksDone = 0;
         p.ctrl->moveTicket = 0;
-        p.ctrl->didSort = p.fuseCopyBack ? 0 : p.hasExported;
+        p.ctrl->didSort = p.hasExported;
     }
 }
 
@@ -650,7 +602,6 @@ sortRearrangeKernel(SortParams p)
 __global__ void __launch_bounds__(256)
 sortCopyBackKernel(SortParams p, unsigned long long exported_mask)
 {
-    pdlSync();
     TableDesc &t = p.state->tables[p.archetype];
     if (!p.ctrl->didSort) return;
     const int32_t n = t.numRows;
@@ -703,12 +654,6 @@ bool sortScratchCreate(Executor *ex, std::string *err)
             max_cap = std::max(max_cap, S.tables[a].capacity);
     }
 
-    auto alloc = [&](void **p, size_t bytes) {
-        if (cudaMalloc(p, bytes) != cudaSuccess) return false;
-        ex->allocations.push_back(*p);
-        cudaMemsetAsync(*p, 0, bytes, ex->stream);
-        return true;
-    };
     // key / index / look-back scratch: address ranges big enough for any table, memory
     // mapped for the largest table that exists (sortScratchEnsure maps more)
     const size_t max_rows = 0x7fffff00ull;
@@ -722,9 +667,9 @@ bool sortScratchCreate(Executor *ex, std::string *err)
     ok = ok && vmReserve(ex->gpu, &sc->lookbackRange, (max_rows / kTileItems + 2) * kMaxPasses * 256 * 4, 4096, err);
     sc->lookback = (uint32_t *)sc->lookbackRange.base;
     if (!ok || !sortScratchEnsure(ex, max_cap, err)) return false;
-    ok = ok && alloc((void **)&sc->bins, sizeof(int32_t) * kMaxPasses * 256);
-    ok = ok && alloc((void **)&sc->ctrl, sizeof(SortCtrl));
-    ok = ok && alloc((void **)&sc->altColumns, sizeof(void *) * kMaxArchetypes * kMaxColumns);
+    ok = ok && devAlloc(ex, (void **)&sc->bins, sizeof(int32_t) * kMaxPasses * 256);
+    ok = ok && devAlloc(ex, (void **)&sc->ctrl, sizeof(SortCtrl));
+    ok = ok && devAlloc(ex, (void **)&sc->altColumns, sizeof(void *) * kMaxArchetypes * kMaxColumns);
     if (!ok) {
         *err = "sort scratch allocation failed";
         return false;
@@ -752,7 +697,7 @@ bool sortScratchCreate(Executor *ex, std::string *err)
                 if (!vmReserve(ex->gpu, &ex->twinRanges[a][c], ex->columnRanges[a][c].reserved,
                                (size_t)t.columnBytes[c] * t.capacity + 256, err)) return false;
                 p = ex->twinRanges[a][c].base;
-            } else if (!alloc(&p, (size_t)t.columnBytes[c] * t.capacity + 256)) {
+            } else if (!devAlloc(ex, &p, (size_t)t.columnBytes[c] * t.capacity + 256)) {
                 *err = "sort twin buffer allocation failed";
                 return false;
             }
@@ -837,39 +782,22 @@ void launchSortArchetype(Executor *ex, uint32_t archetype, int32_t col, cudaStre
         if (sc->exportedMask[archetype][c]) mask |= 1ull << c;
     }
     p.hasExported = mask ? 1 : 0;
-    p.exportedMask = mask;
-    static const int fuse_copy_back = [] {
-        const char *v = getenv("MADRONA_B200_SORT_FUSE_COPYBACK");
-        // B200, sortcheck 3.1M rows, one box: copy-back items fused into the rearrange kernel
-        // 0.458 ms/step, separate copy-back launch 0.442 -> separate by default
-        return (v && *v) ? atoi(v) : 0;
-    }();
-    p.fuseCopyBack = fuse_copy_back && mask ? 1 : 0;
 
     const int tiles = (t.capacity + kTileItems - 1) / kTileItems;
     const int hist_grid = std::max(1, std::min(tiles, ex->numSMs * 4));
-    // ticketed tiles: any grid size is deadlock free; more resident blocks hide the
-    // ranking / look-back latency of each tile
-    static const int sweep_per_sm = [] {
-        const char *v = getenv("MADRONA_B200_SWEEP_BLOCKS_PER_SM");
-        return (v && *v) ? std::max(1, atoi(v)) : 4;   // B200, 3.1M rows: 2 -> 0.659, 3 -> 0.615, 4 -> 0.598, 6 -> 0.599 ms
-    }();
-    const int sweep_grid = std::max(1, std::min(tiles, ex->numSMs * sweep_per_sm));
-    launchK(sortHistogramKernel, dim3(hist_grid), dim3(kSortThreads), 0, s, p);
+    const int sweep_grid = std::max(1, std::min(tiles, ex->numSMs * MB2_SWEEP_BLOCKS_PER_SM));
+    sortHistogramKernel<<<hist_grid, kSortThreads, 0, s>>>(p);
     for (int pass = 0; pass < p.numPasses; pass++) {
-        launchK(sortOnesweepKernel, dim3(sweep_grid), dim3(kSortThreads), 0, s, p, pass);
+        sortOnesweepKernel<<<sweep_grid, kSortThreads, 0, s>>>(p, pass);
     }
     const int rtiles = (t.capacity + kRearrangeTile - 1) / kRearrangeTile;
-    static const int move_per_sm = [] {
-        const char *v = getenv("MADRONA_B200_REARRANGE_BLOCKS_PER_SM");
-        return (v && *v) ? std::max(1, atoi(v)) : 8;
-    }();
-    const int rblocks = std::max(1, std::min(rtiles * std::max(1, t.numColumns / 2), ex->numSMs * move_per_sm));
-    launchK(sortRearrangeKernel, dim3(rblocks), dim3(256), 0, s, p);
+    const int rblocks = std::max(1, std::min(rtiles * std::max(1, t.numColumns / 2),
+                                             ex->numSMs * MB2_REARRANGE_BLOCKS_PER_SM));
+    sortRearrangeKernel<<<rblocks, 256, 0, s>>>(p);
     const int row_blocks = std::max(1, std::min((t.capacity + 255) / 256, ex->numSMs * 4));
     dim3 rgrid((unsigned)row_blocks, (unsigned)t.numColumns);
 
-    if (mask && !p.fuseCopyBack) launchK(sortCopyBackKernel, dim3(rgrid), dim3(256), 0, s, p, mask);
+    if (mask) sortCopyBackKernel<<<rgrid, 256, 0, s>>>(p, mask);
 }
 
 }

@@ -214,13 +214,4 @@ enum ErrorFlags : u32 {
     ErrPhysicsOverflow = 1u << 6,
 };
 
-#ifdef __CUDACC__
-// First statement of every engine / simulator kernel (see engine.hpp launchK).
-__device__ __forceinline__ void pdlSync()
-{
-    asm volatile("griddepcontrol.launch_dependents;");
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-#endif
-
 }

@@ -596,10 +596,6 @@ Entity BVH::traceRay(math::Vector3 o, math::Vector3 d, float *out_hit_t,
     // rejected on B200, room 8192 worlds: seeding t_max with the hit of the nearest-entry leaf
     // before the walk -- 1.091 vs 1.019 ms/step, the extra pass costs more than the leaf tests
     // it saves.)
-#ifndef MB2_TRACE_MASK
-#define MB2_TRACE_MASK 1
-#endif
-#if MB2_TRACE_MASK
     const unsigned peers = __activemask();
     const mb2::PVec4 *boxes = s_.orderedBoxes;
     const int32_t num_boxes = s_.numTraversal;
@@ -651,48 +647,6 @@ Entity BVH::traceRay(math::Vector3 o, math::Vector3 d, float *out_hit_t,
             }
         }
     }
-#else
-    // one-phase scan (the round-2 batch A mechanism), kept for A/B builds
-    const unsigned peers = __activemask();
-    const mb2::PVec4 *boxes = s_.orderedBoxes;
-    const int32_t num_boxes = s_.numTraversal;
-    int32_t k = 0;
-    bool walking = true;
-    Entity closest = Entity::none();
-    math::Vector3 closest_normal { 0, 0, 0 };
-
-    while (__any_sync(peers, walking)) {
-        int32_t leaf_idx = -1;
-        while (walking) {
-            if (k >= num_boxes) {
-                walking = false;
-                break;
-            }
-            const mb2::PVec4 b0 = boxes[2 * k], b1 = boxes[2 * k + 1];
-            k += 1;
-            const float lx = inv_d.d0 * (b0.x - o.x), ux = inv_d.d0 * (b0.w - o.x);
-            const float ly = inv_d.d1 * (b0.y - o.y), uy = inv_d.d1 * (b1.x - o.y);
-            const float lz = inv_d.d2 * (b0.z - o.z), uz = inv_d.d2 * (b1.y - o.z);
-            const float entry = fmaxf(fminf(lx, ux), fmaxf(fminf(ly, uy), fmaxf(fminf(lz, uz), 0.f)));
-            const float exit = fminf(fmaxf(lx, ux), fminf(fmaxf(ly, uy), fminf(fmaxf(lz, uz), t_max)));
-            if (entry <= exit) {
-                leaf_idx = __float_as_int(b1.z);
-                break;
-            }
-        }
-        __syncwarp(peers);
-
-        if (leaf_idx >= 0) {
-            float hit_t;
-            math::Vector3 leaf_normal;
-            if (traceRayIntoLeaf(leaf_idx, o, d, 0.f, t_max, &hit_t, &leaf_normal)) {
-                t_max = hit_t;
-                closest = unpackEntity(s_.leafEntities[leaf_idx]);
-                closest_normal = leaf_normal;
-            }
-        }
-    }
-#endif
     if (closest == Entity::none()) return Entity::none();
     *out_hit_t = t_max;
     *out_hit_normal = closest_normal;

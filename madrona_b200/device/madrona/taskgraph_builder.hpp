@@ -28,7 +28,6 @@ __device__ uint32_t nodeMeta = 0;
 template <typename NodeT>
 __global__ void __launch_bounds__(256) nodeKern(const mb2::NodeRecord *rec)
 {
-    mb2::pdlSync();     // programmatic dependent launch, see csrc/engine.hpp launchK
     NodeT::run(*rec);
 }
 

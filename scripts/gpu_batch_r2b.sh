@@ -1,4 +1,5 @@
 #!/bin/bash
+# (Record only: MADRONA_B200_SORT_FUSE_COPYBACK and the MADRONA_B200_*_BLOCKS_PER_SM switches used below no longer exist.)
 # Round-2 batch B (one gpurun call): parity of the new kernels, bench lines, one-box A/Bs of
 # every switch added since batch A, then ncu captures (last: a killed ncu can wedge a GPU).
 # Variant libraries used below were built beforehand (git-ignored) with

@@ -1,4 +1,5 @@
 #!/bin/bash
+# (Record only: -DMB2_TRACE_MASK=0, MADRONA_B200_SORT_FUSE_COPYBACK and MADRONA_B200_REARRANGE_BLOCKS_PER_SM used below no longer exist.)
 # Round-2 batch C (one gpurun call): parity, one-box A/Bs of the last switches (traceRay candidate
 # mask, ballot digit matching, rearrange residency), then the bench lines and ncu captures of the
 # configuration the A/Bs select (recorded in gpurun_out/r2c_selected.env), ncu last.

@@ -1,12 +1,8 @@
 """Control logic of the sort kernels (madrona_b200/csrc/kernels_sort.cu), modelled on the CPU:
-  * the decoupled look-back of a onesweep tile reads kLookWindow predecessors at a time and
-    consumes them in order (stop at the first unpublished one and retry from it, finish at the
-    first inclusive prefix): it must produce the same exclusive prefix as walking one
-    predecessor at a time, whatever the publication timing;
-  * the rearrange kernel's work items are (phase, chunk) tickets with phases
-    G(col 0) [C(col 0)] G(col 1) ... in column-major order; with fused copy-back a C(col)
-    item may only ever wait for items with SMALLER tickets (that is what makes the spin wait
-    deadlock free for any grid size)."""
+the decoupled look-back of a onesweep tile reads kLookWindow predecessors at a time and
+consumes them in order (stop at the first unpublished one and retry from it, finish at the
+first inclusive prefix): it must produce the same exclusive prefix as walking one
+predecessor at a time, whatever the publication timing."""
 import numpy as np
 
 AGG, INC = 1, 2
@@ -64,35 +60,3 @@ def test_windowed_lookback_equals_serial_walk_under_any_publication_order():
                 return 0, 0
             assert walk(read, tile) == int(incl[tile - 1]), (walk.__name__, tile)
 
-
-def decode(item, chunks, num_cols, fused_mask):
-    phase, chunk = divmod(item, chunks)
-    col = 0
-    while col < num_cols:
-        span = 1 + ((fused_mask >> col) & 1)
-        if phase < span:
-            return col, chunk, phase == 1
-        phase -= span
-        col += 1
-    raise AssertionError("ticket past the last phase")
-
-
-def test_copy_back_items_only_wait_for_smaller_tickets():
-    rng = np.random.default_rng(4)
-    for _ in range(100):
-        num_cols = int(rng.integers(1, 12))
-        chunks = int(rng.integers(1, 9))
-        fused_mask = int(rng.integers(0, 1 << num_cols))
-        num_items = chunks * (num_cols + bin(fused_mask).count("1"))
-        gather_tickets, seen = {}, set()
-        for item in range(num_items):
-            col, chunk, copy_back = decode(item, chunks, num_cols, fused_mask)
-            assert (col, chunk, copy_back) not in seen
-            seen.add((col, chunk, copy_back))
-            if copy_back:
-                assert (fused_mask >> col) & 1
-                # it waits for every gather chunk of its column: all of them were handed out before
-                assert len(gather_tickets[col]) == chunks and max(gather_tickets[col]) < item
-            else:
-                gather_tickets.setdefault(col, []).append(item)
-        assert len(seen) == num_items and set(gather_tickets) == set(range(num_cols))
