@@ -41,86 +41,20 @@ using madrona::math::Mat3x3;
 using madrona::math::AABB;
 using madrona::math::cross;
 using madrona::math::dot;
+using madrona::geo::HalfEdge;
+using madrona::geo::HalfEdgeMesh;
+using madrona::geo::Plane;
+using madrona::phys::CollisionPrimitive;
+using madrona::phys::JointConstraint;
+using madrona::phys::ObjectManager;
+using madrona::phys::PhysicsSystemState;
+using madrona::phys::ResponseType;
+using madrona::phys::RigidBodyMetadata;
+using madrona::phys::Velocity;
+using madrona::phys::xpbd::PreSolvePositional;
+using madrona::phys::xpbd::PreSolveVelocity;
+using madrona::phys::xpbd::SubstepPrevState;
 
-// ---- mirrors of the simulator-facing object description ----------------------
-// (layout == madrona::phys::ObjectManager & friends, device/madrona/physics.hpp)
-struct PHalfEdge {
-    u32 next;
-    u32 rootVertex;
-    u32 face;
-};
-
-struct PPlane {
-    Vector3 normal;
-    float d;
-};
-
-struct PHalfEdgeMesh {
-    PHalfEdge *halfEdges;
-    u32 *faceBaseHalfEdges;
-    PPlane *facePlanes;
-    Vector3 *vertices;
-    u32 numHalfEdges;
-    u32 numFaces;
-    u32 numVertices;
-};
-
-struct PCollisionPrimitive {
-    u32 type;     // 1 sphere, 2 hull, 4 plane
-    union {
-        float sphereRadius;
-        PHalfEdgeMesh hull;
-    };
-};
-
-struct PMetadata {
-    float invMass;
-    Vector3 invInertia;
-    Vector3 toCenterOfMass;
-    Quat toInertiaFrame;
-    float muS;
-    float muD;
-};
-
-struct PObjectManager {
-    PCollisionPrimitive *prims;
-    AABB *primAABBs;
-    AABB *bodyAABBs;
-    u32 *primOffsets;
-    u32 *primCounts;
-    PMetadata *metadata;
-};
-
-static_assert(sizeof(PMetadata) == 52, "RigidBodyMetadata layout");
-static_assert(sizeof(PCollisionPrimitive) == 56, "CollisionPrimitive layout");
-static_assert(sizeof(BVHNode) == 116, "BVH node layout");
-static_assert(sizeof(Contact) == 112, "contact layout");
-static_assert(sizeof(Candidate) == 16, "candidate layout");
-
-struct PVelocity {
-    Vector3 linear;
-    Vector3 angular;
-};
-
-struct PPosRot {        // SubstepPrevState / PreSolvePositional
-    Vector3 x;
-    Quat q;
-};
-
-struct PJoint {         // == phys::JointConstraint (92 bytes)
-    u32 e1Gen; i32 e1ID;
-    u32 e2Gen; i32 e2ID;
-    i32 type;           // 0 fixed, 1 hinge
-    union {
-        struct { Quat attachRot1; Quat attachRot2; float separation; } fixed;
-        struct { Vector3 a1Local, a2Local, b1Local, b2Local; } hinge;
-    };
-    Vector3 r1;
-    Vector3 r2;
-};
-static_assert(sizeof(PJoint) == 92, "JointConstraint layout");
-
-constexpr u32 kRespDynamic = 0, kRespStatic = 2;
 constexpr int kPhysWarps = 2;     // worlds (warps) per block of the per-world physics kernels
 
 struct PhysicsHost {
@@ -131,11 +65,6 @@ struct PhysicsHost {
 };
 
 // ---- small device helpers ------------------------------------------------------------
-
-struct BodyView {
-    const TableDesc *t;
-    const i32 *cols;
-};
 
 __device__ __forceinline__ const BodyArchetype *bodyOf(const PhysicsState &P, u32 arch)
 {
@@ -191,15 +120,15 @@ __device__ __forceinline__ WorldBVH &worldBVH(const EngineState &S, const Physic
     return ((WorldBVH *)S.tables[P.bvhArchetype].columns[2])[w];
 }
 
-__device__ __forceinline__ const PhysicsWorldParams &worldParams(const EngineState &S, const PhysicsState &P, i32 w)
+__device__ __forceinline__ const PhysicsSystemState &worldParams(const EngineState &S, const PhysicsState &P, i32 w)
 {
-    return ((const PhysicsWorldParams *)S.tables[P.paramsArchetype].columns[2])[w];
+    return ((const PhysicsSystemState *)S.tables[P.paramsArchetype].columns[2])[w];
 }
 
-__device__ __forceinline__ const PObjectManager &worldObjects(const EngineState &S, const PhysicsState &P, i32 w)
+__device__ __forceinline__ const ObjectManager &worldObjects(const EngineState &S, const PhysicsState &P, i32 w)
 {
-    return **(const PObjectManager *const *)((const char *)S.tables[P.objectDataArchetype].columns[2] +
-                                             (size_t)w * 8);
+    return **(const ObjectManager *const *)((const char *)S.tables[P.objectDataArchetype].columns[2] +
+                                            (size_t)w * 8);
 }
 
 __device__ __forceinline__ Vector3 mulDiag(Vector3 d, Vector3 v)
@@ -279,23 +208,20 @@ __device__ __forceinline__ void rowUpdateLeaf(const EngineState &S, const Physic
 {
     {
         WorldBVH &bvh = worldBVH(S, P, w);
-        const PObjectManager &objs = *(const PObjectManager *)bvh.objMgr;
+        const ObjectManager &objs = *bvh.objMgr;
 
         const i32 leaf = bodyCol<i32>(S, b, PCLeafID, row);
         const Vector3 pos = bodyCol<Vector3>(S, b, PCPosition, row);
         const Quat rot = loadQuat(&bodyCol<Quat>(S, b, PCRotation, row));
         const Diag3x3 scale = bodyCol<Diag3x3>(S, b, PCScale, row);
         const i32 obj = bodyCol<i32>(S, b, PCObjectID, row);
-        const Vector3 lin_vel = bodyCol<PVelocity>(S, b, PCVelocity, row).linear;
+        const Vector3 lin_vel = bodyCol<Velocity>(S, b, PCVelocity, row).linear;
 
-        AABB world_box = objs.bodyAABBs[obj].applyTRS(pos, rot, scale);
+        AABB world_box = objs.rigidBodyAABBs[obj].applyTRS(pos, rot, scale);
         AABB grown = growByMotion(world_box, lin_vel, bvh.velExpansion, bvh.accelExpansion);
 
-        PAABB out { { grown.pMin.x, grown.pMin.y, grown.pMin.z },
-                    { grown.pMax.x, grown.pMax.y, grown.pMax.z } };
-        storePairs(&bvh.leafAABBs[leaf], out);
-        LeafTransform lt { { pos.x, pos.y, pos.z }, { rot.w, rot.x, rot.y, rot.z },
-                           { scale.d0, scale.d1, scale.d2 } };
+        storePairs(&bvh.leafAABBs[leaf], grown);
+        LeafTransform lt { pos, rot, { scale.d0, scale.d1, scale.d2 } };
         storePairs(&bvh.leafTransforms[leaf], lt);
         bvh.sortedLeaves[leaf] = leaf;
     }
@@ -305,10 +231,8 @@ __device__ __forceinline__ void rowUpdateLeaf(const EngineState &S, const Physic
 
 __device__ __forceinline__ Vector3 leafCenter(const WorldBVH &bvh, i32 slot)
 {
-    const PAABB &b = bvh.leafAABBs[bvh.sortedLeaves[slot]];
-    Vector3 lo { b.pMin.x, b.pMin.y, b.pMin.z };
-    Vector3 hi { b.pMax.x, b.pMax.y, b.pMax.z };
-    return (lo + hi) / 2.f;
+    const AABB b = bvh.leafAABBs[bvh.sortedLeaves[slot]];
+    return (b.pMin + b.pMax) / 2.f;
 }
 
 // Partition sortedLeaves[base, base+n) around the midpoint of the centroid
@@ -373,7 +297,7 @@ __device__ void rebuildWorldBVH(WorldBVH &bvh)
             for (int i = 0; i < 4; i++) {
                 if (i < top.count) {
                     i32 leaf = bvh.sortedLeaves[top.offset + i];
-                    const PAABB box = bvh.leafAABBs[leaf];
+                    const AABB box = bvh.leafAABBs[leaf];
                     bvh.leafParents[leaf] = ((u32)node_id << 2) | (u32)i;
                     node.children[i] = (i32)(0x80000000u | (u32)leaf);
                     node.minX[i] = box.pMin.x; node.minY[i] = box.pMin.y; node.minZ[i] = box.pMin.z;
@@ -482,7 +406,7 @@ __device__ __forceinline__ void phaseRebuild(const EngineState &S, const Physics
 // ancestors while something actually grew (broadphase.cpp:550-647).
 __device__ void refitLeaf(WorldBVH &bvh, i32 leaf)
 {
-    const PAABB box = bvh.leafAABBs[leaf];
+    const AABB box = bvh.leafAABBs[leaf];
     const u32 packed = bvh.leafParents[leaf];
     i32 node_idx = (i32)(packed >> 2);
     const int sub = (int)(packed & 3u);
@@ -554,7 +478,7 @@ constexpr u32 kUnknownSlot = 0x7fffu;
 struct PairVisitor {
     const EngineState &S;
     const PhysicsState &P;
-    const PObjectManager &objs;
+    const ObjectManager &objs;
     i32 selfID;
     bool selfStatic;
     u32 selfPrims;
@@ -590,8 +514,9 @@ __device__ __forceinline__ void forEachPartner(const WorldBVH &bvh, const PairVi
                 const i32 b_row = slot.b;
                 const BodyArchetype *bb = bodyOf(v.P, b_arch);
                 if (!bb) continue;
-                if (v.selfStatic && bodyCol<u32>(v.S, *bb, PCResponseType, b_row) == kRespStatic) continue;
-                const u32 b_prims = v.objs.primCounts[bodyCol<i32>(v.S, *bb, PCObjectID, b_row)];
+                if (v.selfStatic &&
+                    bodyCol<ResponseType>(v.S, *bb, PCResponseType, b_row) == ResponseType::Static) continue;
+                const u32 b_prims = v.objs.rigidBodyPrimitiveCounts[bodyCol<i32>(v.S, *bb, PCObjectID, b_row)];
                 fn(b_arch, b_row, b_prims);
             } else if (depth < 32) {
                 stack[depth++] = child;
@@ -627,7 +552,7 @@ __device__ void phaseFindCandidates(EngineState &S, const PhysicsState &P, const
                                     const int warp, CandidateScratch &scratch)
 {
     const WorldBVH &bvh = worldBVH(S, P, w);
-    const PObjectManager &objs = *(const PObjectManager *)bvh.objMgr;
+    const ObjectManager &objs = *bvh.objMgr;
     Candidate *out = P.candidates + (size_t)w * P.maxCandidatesPerWorld;
     StagedLeaf *staged = scratch.leaves[warp];
     i32 running = 0;
@@ -675,8 +600,8 @@ __device__ void phaseFindCandidates(EngineState &S, const PhysicsState &P, const
             if (bb) {
                 sl.arch = (u32)es.a;
                 sl.row = es.b;
-                sl.isStatic = bodyCol<u32>(S, *bb, PCResponseType, es.b) == kRespStatic ? 1u : 0u;
-                sl.prims = objs.primCounts[bodyCol<i32>(S, *bb, PCObjectID, es.b)];
+                sl.isStatic = bodyCol<ResponseType>(S, *bb, PCResponseType, es.b) == ResponseType::Static ? 1u : 0u;
+                sl.prims = objs.rigidBodyPrimitiveCounts[bodyCol<i32>(S, *bb, PCObjectID, es.b)];
                 sl.slotInfo = bodySlotInfo(sl.arch, sl.row, sl.isStatic != 0);
                 if (sl.arch > 0xffu || sl.prims > 0xffu) {
                     atomicOr(&S.errorFlags, (u32)ErrPhysicsOverflow);   // does not fit the packed candidate
@@ -705,15 +630,14 @@ __device__ void phaseFindCandidates(EngineState &S, const PhysicsState &P, const
             if (valid) {
                 const u64 packed = ((const u64 *)t.columns[0])[row];
                 self_id = (i32)(u32)(packed >> 32);
-                self_static = bodyCol<u32>(S, b, PCResponseType, row) == kRespStatic;
-                self_prims = objs.primCounts[bodyCol<i32>(S, b, PCObjectID, row)];
+                self_static = bodyCol<ResponseType>(S, b, PCResponseType, row) == ResponseType::Static;
+                self_prims = objs.rigidBodyPrimitiveCounts[bodyCol<i32>(S, b, PCObjectID, row)];
                 self_info = bodySlotInfo(b.archetype, row, self_static);
                 if (b.archetype > 0xffu || self_prims > 0xffu) {
                     atomicOr(&S.errorFlags, (u32)ErrPhysicsOverflow);
                     self_prims = 0;
                 }
-                const PAABB lb = bvh.leafAABBs[bodyCol<i32>(S, b, PCLeafID, row)];
-                box = AABB { { lb.pMin.x, lb.pMin.y, lb.pMin.z }, { lb.pMax.x, lb.pMax.y, lb.pMax.z } };
+                box = bvh.leafAABBs[bodyCol<i32>(S, b, PCLeafID, row)];
             }
 
             // stage 2: which staged leaves does this body pair with (bit k of word k / 64)
@@ -783,35 +707,35 @@ __device__ __forceinline__ void rowIntegrate(const EngineState &S, const Physics
 
         Vector3 x = bodyCol<Vector3>(S, b, PCPosition, row);
         Quat q = loadQuat(&bodyCol<Quat>(S, b, PCRotation, row));
-        const PVelocity vel = loadPairs(&bodyCol<PVelocity>(S, b, PCVelocity, row));
+        const Velocity vel = loadPairs(&bodyCol<Velocity>(S, b, PCVelocity, row));
         Vector3 v = vel.linear;
         Vector3 omega = vel.angular;
-        const u32 resp = bodyCol<u32>(S, b, PCResponseType, row);
+        const ResponseType resp = bodyCol<ResponseType>(S, b, PCResponseType, row);
 
-        PPosRot &prev = bodyCol<PPosRot>(S, b, PCPrevState, row);
-        PPosRot &pre_pos = bodyCol<PPosRot>(S, b, PCPreSolvePos, row);
-        PVelocity &pre_vel = bodyCol<PVelocity>(S, b, PCPreSolveVel, row);
+        SubstepPrevState &prev = bodyCol<SubstepPrevState>(S, b, PCPrevState, row);
+        PreSolvePositional &pre_pos = bodyCol<PreSolvePositional>(S, b, PCPreSolvePos, row);
+        PreSolveVelocity &pre_vel = bodyCol<PreSolveVelocity>(S, b, PCPreSolveVel, row);
 
-        prev.x = x;
-        prev.q = q;
-        if (resp == kRespStatic) {
+        prev.prevPosition = x;
+        prev.prevRotation = q;
+        if (resp == ResponseType::Static) {
             pre_pos.x = x;
             pre_pos.q = q;
-            storePairs(&pre_vel, PVelocity { Vector3::zero(), Vector3::zero() });
+            storePairs(&pre_vel, PreSolveVelocity { Vector3::zero(), Vector3::zero() });
             return;
         }
 
-        const PhysicsWorldParams &params = worldParams(S, P, w);
-        const PObjectManager &objs = worldObjects(S, P, w);
-        const PMetadata &meta = objs.metadata[bodyCol<i32>(S, b, PCObjectID, row)];
-        const float inv_m = meta.invMass;
-        const Vector3 inv_I = meta.invInertia;
+        const PhysicsSystemState &params = worldParams(S, P, w);
+        const ObjectManager &objs = worldObjects(S, P, w);
+        const RigidBodyMetadata &meta = objs.metadata[bodyCol<i32>(S, b, PCObjectID, row)];
+        const float inv_m = meta.mass.invMass;
+        const Vector3 inv_I = meta.mass.invInertiaTensor;
         const float h = params.h;
         const Vector3 g { params.g.x, params.g.y, params.g.z };
         const Vector3 ext_force = bodyCol<Vector3>(S, b, PCExtForce, row);
         const Vector3 ext_torque = bodyCol<Vector3>(S, b, PCExtTorque, row);
 
-        if (resp == kRespDynamic) v += h * g;
+        if (resp == ResponseType::Dynamic) v += h * g;
         v += h * inv_m * ext_force;
         x += h * v;
 
@@ -834,28 +758,28 @@ __device__ __forceinline__ void rowIntegrate(const EngineState &S, const Physics
         storeQuat(&bodyCol<Quat>(S, b, PCRotation, row), q);
         pre_pos.x = x;
         pre_pos.q = q;
-        storePairs(&pre_vel, PVelocity { v, omega });
+        storePairs(&pre_vel, PreSolveVelocity { v, omega });
     }
 }
 
 // ---- TGS (src/physics/tgs.cpp): the reference's solver skeleton integrates and nothing else
 __device__ __forceinline__ void rowTGSVelocities(const EngineState &S, const PhysicsState &P, const BodyArchetype &b, const i32 row, const i32 w)
 {
-    const u32 resp = bodyCol<u32>(S, b, PCResponseType, row);
-    if (resp == kRespStatic) return;
-    PVelocity &vel_ref = bodyCol<PVelocity>(S, b, PCVelocity, row);
-    const PVelocity vel = loadPairs(&vel_ref);
+    const ResponseType resp = bodyCol<ResponseType>(S, b, PCResponseType, row);
+    if (resp == ResponseType::Static) return;
+    Velocity &vel_ref = bodyCol<Velocity>(S, b, PCVelocity, row);
+    const Velocity vel = loadPairs(&vel_ref);
     Vector3 v = vel.linear;
     Vector3 omega = vel.angular;
     const Quat q = loadQuat(&bodyCol<Quat>(S, b, PCRotation, row));
-    const PhysicsWorldParams &params = worldParams(S, P, w);
-    const PObjectManager &objs = worldObjects(S, P, w);
-    const PMetadata &meta = objs.metadata[bodyCol<i32>(S, b, PCObjectID, row)];
-    const float inv_m = meta.invMass;
-    const Vector3 inv_I = meta.invInertia;
+    const PhysicsSystemState &params = worldParams(S, P, w);
+    const ObjectManager &objs = worldObjects(S, P, w);
+    const RigidBodyMetadata &meta = objs.metadata[bodyCol<i32>(S, b, PCObjectID, row)];
+    const float inv_m = meta.mass.invMass;
+    const Vector3 inv_I = meta.mass.invInertiaTensor;
     const float h = params.h;
     const Vector3 g { params.g.x, params.g.y, params.g.z };
-    if (resp == kRespDynamic) v += h * g;
+    if (resp == ResponseType::Dynamic) v += h * g;
     v += h * inv_m * bodyCol<Vector3>(S, b, PCExtForce, row);
     const Vector3 I { inv_I.x == 0 ? 0.0f : 1.0f / inv_I.x,
                       inv_I.y == 0 ? 0.0f : 1.0f / inv_I.y,
@@ -866,7 +790,7 @@ __device__ __forceinline__ void rowTGSVelocities(const EngineState &S, const Phy
     // NB: the reference multiplies I by the WORLD-space omega here (tgs.cpp:133-134)
     omega_local += h * mulDiag(inv_I, tau_local - cross(omega_local, mulDiag(I, omega)));
     omega = q.rotateVec(omega_local);
-    storePairs(&vel_ref, PVelocity { v, omega });
+    storePairs(&vel_ref, Velocity { v, omega });
 }
 
 __device__ __forceinline__ void rowTGSPositions(const EngineState &S, const PhysicsState &P, const BodyArchetype &b, const i32 row, const i32 w)
@@ -874,7 +798,7 @@ __device__ __forceinline__ void rowTGSPositions(const EngineState &S, const Phys
     const float h = worldParams(S, P, w).h;
     Vector3 x = bodyCol<Vector3>(S, b, PCPosition, row);
     Quat q = loadQuat(&bodyCol<Quat>(S, b, PCRotation, row));
-    const PVelocity vel = loadPairs(&bodyCol<PVelocity>(S, b, PCVelocity, row));
+    const Velocity vel = loadPairs(&bodyCol<Velocity>(S, b, PCVelocity, row));
     x += h * vel.linear;
     const Quat spin = Quat::fromAngularVec(0.5f * h * vel.angular);
     q += spin * q;
@@ -889,21 +813,22 @@ __device__ __forceinline__ void rowSetVelocity(const EngineState &S, const Physi
         const float h = worldParams(S, P, w).h;
         const Vector3 x = bodyCol<Vector3>(S, b, PCPosition, row);
         const Quat q = loadQuat(&bodyCol<Quat>(S, b, PCRotation, row));
-        const PPosRot prev = bodyCol<PPosRot>(S, b, PCPrevState, row);
+        const SubstepPrevState prev = bodyCol<SubstepPrevState>(S, b, PCPrevState, row);
 
         // bitwise-equal orientations mean exactly zero angular velocity
         Quat dq;
-        if (q.w != prev.q.w || q.x != prev.q.x || q.y != prev.q.y || q.z != prev.q.z) {
-            dq = q * prev.q.inv();
+        if (q.w != prev.prevRotation.w || q.x != prev.prevRotation.x ||
+            q.y != prev.prevRotation.y || q.z != prev.prevRotation.z) {
+            dq = q * prev.prevRotation.inv();
         } else {
             dq = Quat { 1, 0, 0, 0 };
         }
         const Vector3 new_omega = 2.f / h * Vector3 { dq.x, dq.y, dq.z };
 
-        PVelocity out;
-        out.linear = (x - prev.x) / h;
+        Velocity out;
+        out.linear = (x - prev.prevPosition) / h;
         out.angular = dq.w > 0.f ? new_omega : -new_omega;
-        storePairs(&bodyCol<PVelocity>(S, b, PCVelocity, row), out);
+        storePairs(&bodyCol<Velocity>(S, b, PCVelocity, row), out);
     }
 }
 
@@ -912,9 +837,9 @@ __device__ __forceinline__ void rowSetVelocity(const EngineState &S, const Physi
 // =============================================================================================
 
 struct HullInWorld {
-    const PHalfEdgeMesh *mesh;
+    const HalfEdgeMesh *mesh;
     Vector3 *verts;     // world space
-    PPlane *planes;     // world space
+    Plane *planes;      // world space
     u32 numVerts;
     u32 numFaces;
     Vector3 center;
@@ -923,12 +848,12 @@ struct HullInWorld {
 // (placement: vertex = R S v + t, normal = normalize(R S^-1 n), plane offset through a
 // transformed point of the plane, centre = vertex mean -- narrowphase.cpp:151-223;
 // done by the lanes of the warp in hullHullCooperative, on the fly for hull-plane)
-__device__ __forceinline__ float planeDistance(const PPlane &pl, Vector3 p)
+__device__ __forceinline__ float planeDistance(const Plane &pl, Vector3 p)
 {
     return dot(p, pl.normal) - pl.d;
 }
 
-__device__ float hullSupportDistance(const PPlane &pl, const HullInWorld &h)
+__device__ float hullSupportDistance(const Plane &pl, const HullInWorld &h)
 {
     float lowest = FLT_MAX;
 #pragma unroll 1
@@ -942,16 +867,16 @@ __device__ float hullSupportDistance(const PPlane &pl, const HullInWorld &h)
 struct FaceAxis {
     float separation;
     i32 face;
-    PPlane plane;
+    Plane plane;
 };
 
 // faces of a against b: ascending, strictly greater wins, stop at the first
 // positive separation (narrowphase.cpp:339-365)
 __device__ FaceAxis bestFaceAxis(const HullInWorld &a, const HullInWorld &b)
 {
-    FaceAxis best { -FLT_MAX, -1, PPlane { Vector3::zero(), 0.f } };
+    FaceAxis best { -FLT_MAX, -1, Plane { Vector3::zero(), 0.f } };
     for (u32 f = 0; f < a.numFaces; f++) {
-        PPlane pl = a.planes[f];
+        Plane pl = a.planes[f];
         float sep = hullSupportDistance(pl, b);
         if (sep > best.separation) {
             best.separation = sep;
@@ -990,14 +915,14 @@ __device__ EdgeAxis bestEdgeAxis(const HullInWorld &a, const HullInWorld &b)
     const u32 ea = a.mesh->numHalfEdges / 2, eb = b.mesh->numHalfEdges / 2;
     for (u32 ia = 0; ia < ea; ia++) {
         const u32 ha = ia * 2;
-        const PHalfEdge a0 = a.mesh->halfEdges[ha];
-        const PHalfEdge a1 = a.mesh->halfEdges[ha ^ 1u];
+        const HalfEdge a0 = a.mesh->halfEdges[ha];
+        const HalfEdge a1 = a.mesh->halfEdges[ha ^ 1u];
         const Vector3 an0 = a.planes[a0.face].normal;
         const Vector3 an1 = a.planes[a1.face].normal;
         for (u32 ib = 0; ib < eb; ib++) {
             const u32 hb = ib * 2;
-            const PHalfEdge b0 = b.mesh->halfEdges[hb];
-            const PHalfEdge b1 = b.mesh->halfEdges[hb ^ 1u];
+            const HalfEdge b0 = b.mesh->halfEdges[hb];
+            const HalfEdge b1 = b.mesh->halfEdges[hb ^ 1u];
             const Vector3 bn0 = b.planes[b0.face].normal;
             const Vector3 bn1 = b.planes[b1.face].normal;
 
@@ -1045,7 +970,7 @@ __device__ i32 mostOpposedFace(const HullInWorld &h, Vector3 ref_normal)
 }
 
 // Sutherland-Hodgman against one plane; "<= 0" is inside (narrowphase.cpp:617-652)
-__device__ __noinline__ int clipAgainst(Vector3 *dst, const PPlane &pl, const Vector3 *src, int n)
+__device__ __noinline__ int clipAgainst(Vector3 *dst, const Plane &pl, const Vector3 *src, int n)
 {
     int m = 0;
     Vector3 v1 = src[n - 1];
@@ -1175,7 +1100,7 @@ __device__ __forceinline__ ManifoldOut reduceManifold(Vector3 normal, const Vect
 
 constexpr int kClipCap = kMaxFaceVerts * 2 + 4;
 
-__device__ ManifoldOut faceFaceManifold(const PPlane &ref_plane, i32 ref_face, i32 inc_face,
+__device__ ManifoldOut faceFaceManifold(const Plane &ref_plane, i32 ref_face, i32 inc_face,
                                         const HullInWorld &ref, const HullInWorld &inc,
                                         Vector3 *buf_a, Vector3 *buf_b)
 {
@@ -1185,7 +1110,7 @@ __device__ ManifoldOut faceFaceManifold(const PPlane &ref_plane, i32 ref_face, i
         u32 he = inc.mesh->faceBaseHalfEdges[inc_face];
         const u32 start = he;
         do {
-            const PHalfEdge cur = inc.mesh->halfEdges[he];
+            const HalfEdge cur = inc.mesh->halfEdges[he];
             he = cur.next;
             if (n < kClipCap) buf_a[n++] = inc.verts[cur.rootVertex];
         } while (he != start);
@@ -1200,7 +1125,7 @@ __device__ ManifoldOut faceFaceManifold(const PPlane &ref_plane, i32 ref_face, i
             he = ref.mesh->halfEdges[he].next;
             Vector3 next_pt = ref.verts[ref.mesh->halfEdges[he].rootVertex];
             Vector3 side_n = cross(next_pt - cur_pt, ref_plane.normal);
-            PPlane side { side_n, dot(side_n, cur_pt) };
+            Plane side { side_n, dot(side_n, cur_pt) };
             cur_pt = next_pt;
             n = n > 0 ? clipAgainst(dst, side, src, n) : 0;
             if (n > kClipCap) n = kClipCap;
@@ -1260,7 +1185,7 @@ __device__ __forceinline__ void writeContact(Contact &c, u32 ref_arch, i32 ref_r
         c.points[i][3] = m.depths[i];
     }
     c.numPoints = m.count;
-    c.normal = PVec3 { m.normal.x, m.normal.y, m.normal.z };
+    c.normal = m.normal;
     c.lambdaN = 0.f;
     c.level = 0;
 }
@@ -1296,7 +1221,7 @@ struct PairSetup {
     u32 aArch, bArch;
     i32 aRow, bRow;
     u32 aInfo, bInfo;  // (world body slot << 1) | mutable, see Candidate::slots
-    const PCollisionPrimitive *aPrim, *bPrim;
+    const CollisionPrimitive *aPrim, *bPrim;
     Vector3 aPos, bPos;
     Quat aRot, bRot;
     Diag3x3 aScale, bScale;
@@ -1305,22 +1230,24 @@ struct PairSetup {
 
 template <bool REJECT>
 __device__ __forceinline__ PairSetup setupPairImpl(const EngineState &S, const PhysicsState &P,
-                                                   const PObjectManager &objs, const Candidate &cand)
+                                                   const ObjectManager &objs, const Candidate &cand)
 {
     PairSetup ps;
     ps.aArch = cand.archPrim & 0xffu; ps.bArch = (cand.archPrim >> 8) & 0xffu;
     ps.aRow = cand.aRow; ps.bRow = cand.bRow;
     ps.aInfo = cand.slots & 0xffffu; ps.bInfo = cand.slots >> 16;
-    u32 a_prim_idx = objs.primOffsets[locCol<i32>(S, P, ps.aArch, ps.aRow, PCObjectID)] + ((cand.archPrim >> 16) & 0xffu);
-    u32 b_prim_idx = objs.primOffsets[locCol<i32>(S, P, ps.bArch, ps.bRow, PCObjectID)] + (cand.archPrim >> 24);
-    ps.aPrim = &objs.prims[a_prim_idx];
-    ps.bPrim = &objs.prims[b_prim_idx];
-    u32 ta = ps.aPrim->type, tb = ps.bPrim->type;
+    u32 a_prim_idx = objs.rigidBodyPrimitiveOffsets[locCol<i32>(S, P, ps.aArch, ps.aRow, PCObjectID)] +
+                     ((cand.archPrim >> 16) & 0xffu);
+    u32 b_prim_idx = objs.rigidBodyPrimitiveOffsets[locCol<i32>(S, P, ps.bArch, ps.bRow, PCObjectID)] +
+                     (cand.archPrim >> 24);
+    ps.aPrim = &objs.collisionPrimitives[a_prim_idx];
+    ps.bPrim = &objs.collisionPrimitives[b_prim_idx];
+    u32 ta = (u32)ps.aPrim->type, tb = (u32)ps.bPrim->type;
     // order the pair by primitive type: sphere(1) < hull(2) < plane(4)
     if (ta > tb) {
         u32 tu;
         i32 ti;
-        const PCollisionPrimitive *tp;
+        const CollisionPrimitive *tp;
         tu = ps.aArch; ps.aArch = ps.bArch; ps.bArch = tu;
         ti = ps.aRow; ps.aRow = ps.bRow; ps.bRow = ti;
         tu = ps.aInfo; ps.aInfo = ps.bInfo; ps.bInfo = tu;
@@ -1336,8 +1263,8 @@ __device__ __forceinline__ PairSetup setupPairImpl(const EngineState &S, const P
     ps.bScale = locCol<Diag3x3>(S, P, ps.bArch, ps.bRow, PCScale);
 
     if constexpr (REJECT) {
-        AABB a_box = objs.primAABBs[a_prim_idx].applyTRS(ps.aPos, ps.aRot, ps.aScale);
-        AABB b_box = objs.primAABBs[b_prim_idx].applyTRS(ps.bPos, ps.bRot, ps.bScale);
+        AABB a_box = objs.primitiveAABBs[a_prim_idx].applyTRS(ps.aPos, ps.aRot, ps.aScale);
+        AABB b_box = objs.primitiveAABBs[b_prim_idx].applyTRS(ps.bPos, ps.bRot, ps.bScale);
         ps.test = a_box.intersects(b_box) ? (ta | tb) : 0u;
     } else {
         ps.test = ta | tb;
@@ -1346,7 +1273,7 @@ __device__ __forceinline__ PairSetup setupPairImpl(const EngineState &S, const P
 }
 
 __device__ __forceinline__ PairSetup setupPair(const EngineState &S, const PhysicsState &P,
-                                               const PObjectManager &objs, const Candidate &cand)
+                                               const ObjectManager &objs, const Candidate &cand)
 {
     return setupPairImpl<true>(S, P, objs, cand);
 }
@@ -1366,9 +1293,9 @@ struct SphereHullResult {
 
 __device__ __noinline__ SphereHullResult sphereHullContact(Vector3 a_pos, float radius, Vector3 b_pos,
                                                            Quat b_rot, Diag3x3 b_scale,
-                                                           const PHalfEdgeMesh *mesh)
+                                                           const HalfEdgeMesh *mesh)
 {
-    const PHalfEdgeMesh &bm = *mesh;
+    const HalfEdgeMesh &bm = *mesh;
     SphereHullResult res { Vector3::zero(), Vector3::zero(), 0.f, 0 };
     if (bm.numVertices > (u32)kMaxHullVerts) {
         res.hit = -1;
@@ -1394,7 +1321,7 @@ __device__ __noinline__ SphereHullResult sphereHullContact(Vector3 a_pos, float 
         Vector3 sep_normal = Vector3::zero();
 #pragma unroll 1
         for (u32 f = 0; f < bm.numFaces; f++) {
-            const PPlane local = bm.facePlanes[f];
+            const Plane local = bm.facePlanes[f];
             const Vector3 on_plane = vert_m * (local.normal * local.d) + hull_origin;
             const Vector3 n = (norm_m * local.normal).normalize();
             const float face_dist = -dot(n, on_plane);
@@ -1424,8 +1351,8 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
 {
     switch (ps.test) {
     case 1: {
-        const float ra = ps.aScale.d0 * ps.aPrim->sphereRadius;
-        const float rb = ps.bScale.d0 * ps.bPrim->sphereRadius;
+        const float ra = ps.aScale.d0 * ps.aPrim->sphere.radius;
+        const float rb = ps.bScale.d0 * ps.bPrim->sphere.radius;
         const Vector3 to_b = ps.bPos - ps.aPos;
         const float dist = to_b.length();
         if (dist > ra + rb) return false;
@@ -1436,7 +1363,7 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
         return true;
     }
     case 5: {
-        const float ra = ps.aScale.d0 * ps.aPrim->sphereRadius;
+        const float ra = ps.aScale.d0 * ps.aPrim->sphere.radius;
         const Vector3 n = ps.bRot.rotateVec(Vector3 { 0, 0, 1 });
         const float d = n.dot(ps.bPos);
         const float t = n.dot(ps.aPos) - d;
@@ -1449,12 +1376,12 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
         // The hull is never stored: every world-space vertex / face normal is
         // produced where it is consumed, with placeHull's per-element formulas
         // (vertex = R S v + t, normal = normalize(R S^-1 n)).
-        const PHalfEdgeMesh &am = ps.aPrim->hull;
+        const HalfEdgeMesh &am = ps.aPrim->hull.halfEdgeMesh;
         const Mat3x3 rot = Mat3x3::fromQuat(ps.aRot);
         const Mat3x3 vert_m = rot * ps.aScale;
         const Mat3x3 norm_m = rot * ps.aScale.inv();
         const Vector3 n = ps.bRot.rotateVec(Vector3 { 0, 0, 1 });
-        const PPlane plane { n, dot(n, ps.bPos) };
+        const Plane plane { n, dot(n, ps.bPos) };
 
         float lowest = FLT_MAX;                       // hullSupportDistance
 #pragma unroll 2
@@ -1483,7 +1410,7 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
         u32 he = am.faceBaseHalfEdges[inc_face];
         const u32 start = he;
         do {
-            const PHalfEdge cur = am.halfEdges[he];
+            const HalfEdge cur = am.halfEdges[he];
             he = cur.next;
             const Vector3 p = vert_m * am.vertices[cur.rootVertex] + ps.aPos;
             const float d = planeDistance(plane, p);
@@ -1500,8 +1427,8 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
     }
     case 3: {
         if constexpr (SPHERE_HULL) {
-            const SphereHullResult r = sphereHullContact(ps.aPos, ps.aScale.d0 * ps.aPrim->sphereRadius,
-                                                         ps.bPos, ps.bRot, ps.bScale, &ps.bPrim->hull);
+            const SphereHullResult r = sphereHullContact(ps.aPos, ps.aScale.d0 * ps.aPrim->sphere.radius,
+                                                         ps.bPos, ps.bRot, ps.bScale, &ps.bPrim->hull.halfEdgeMesh);
             if (r.hit < 0) atomicOr(&S.errorFlags, (u32)ErrPhysicsOverflow);
             if (r.hit <= 0) return false;
             writeContact(out, ps.bArch, ps.bRow, ps.aArch, ps.aRow, singlePoint(r.point, r.normal, r.depth));
@@ -1521,7 +1448,7 @@ __device__ bool narrowphaseSimple(EngineState &S, const PairSetup &ps, Contact &
 
 struct HullScratch {
     Vector3 verts[2 * kMaxHullVerts];
-    PPlane planes[2 * kMaxHullFaces];
+    Plane planes[2 * kMaxHullFaces];
     Vector3 clipA[kClipCap];
     Vector3 clipB[kClipCap];
 };
@@ -1586,7 +1513,7 @@ __device__ __forceinline__ Winner groupSequentialWinner(unsigned gm, float sep, 
 
 // faces of one hull against the other hull's vertices: lane `sub` measures faces
 // sub, sub + 8, ... in ascending order with the scalar rule, then the group combines
-__device__ __forceinline__ Winner groupFaceQuery(unsigned gm, int sub, const PPlane *planes, u32 num_faces,
+__device__ __forceinline__ Winner groupFaceQuery(unsigned gm, int sub, const Plane *planes, u32 num_faces,
                                                  const HullInWorld &other)
 {
     float best = -FLT_MAX;
@@ -1611,8 +1538,8 @@ __device__ __forceinline__ Winner groupFaceQuery(unsigned gm, int sub, const PPl
 __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &scratch, const unsigned gm,
                               const int sub, Contact &out)
 {
-    const PHalfEdgeMesh &am = ps.aPrim->hull;
-    const PHalfEdgeMesh &bm = ps.bPrim->hull;
+    const HalfEdgeMesh &am = ps.aPrim->hull.halfEdgeMesh;
+    const HalfEdgeMesh &bm = ps.bPrim->hull.halfEdgeMesh;
     const u32 nva = am.numVertices, nvb = bm.numVertices, nfa = am.numFaces, nfb = bm.numFaces;
     if (nva > (u32)kMaxHullVerts || nvb > (u32)kMaxHullVerts ||
             nfa > (u32)kMaxHullFaces || nfb > (u32)kMaxHullFaces) {
@@ -1622,7 +1549,7 @@ __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &
 
     // -- both hulls into shared memory (vertex = R S v + t, plane via R S^-1)
     Vector3 *verts_a = scratch.verts, *verts_b = scratch.verts + kMaxHullVerts;
-    PPlane *planes_a = scratch.planes, *planes_b = scratch.planes + kMaxHullFaces;
+    Plane *planes_a = scratch.planes, *planes_b = scratch.planes + kMaxHullFaces;
     {
         const Mat3x3 rot_a = Mat3x3::fromQuat(ps.aRot), rot_b = Mat3x3::fromQuat(ps.bRot);
         const Mat3x3 vm_a = rot_a * ps.aScale, vm_b = rot_b * ps.bScale;
@@ -1636,12 +1563,12 @@ __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &
 #pragma unroll 1
         for (u32 i = (u32)sub; i < nfa + nfb; i += kGroupLanes) {
             const bool is_a = i < nfa;
-            const PPlane local = is_a ? am.facePlanes[i] : bm.facePlanes[i - nfa];
+            const Plane local = is_a ? am.facePlanes[i] : bm.facePlanes[i - nfa];
             const Mat3x3 &vm = is_a ? vm_a : vm_b;
             const Mat3x3 &nm = is_a ? nm_a : nm_b;
             const Vector3 on_plane = vm * (local.normal * local.d) + (is_a ? a_pos : b_pos);
             const Vector3 n = (nm * local.normal).normalize();
-            (is_a ? planes_a[i] : planes_b[i - nfa]) = PPlane { n, dot(n, on_plane) };
+            (is_a ? planes_a[i] : planes_b[i - nfa]) = Plane { n, dot(n, on_plane) };
         }
     }
     __syncwarp(gm);
@@ -1670,10 +1597,10 @@ __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &
 #pragma unroll 1
     for (u32 p = (u32)sub; p < ea * eb; p += kGroupLanes) {
         const u32 ha = (p / eb) * 2, hb = (p % eb) * 2;
-        const PHalfEdge a0 = am.halfEdges[ha];
-        const PHalfEdge a1 = am.halfEdges[ha ^ 1u];
-        const PHalfEdge b0 = bm.halfEdges[hb];
-        const PHalfEdge b1 = bm.halfEdges[hb ^ 1u];
+        const HalfEdge a0 = am.halfEdges[ha];
+        const HalfEdge a1 = am.halfEdges[ha ^ 1u];
+        const HalfEdge b0 = bm.halfEdges[hb];
+        const HalfEdge b1 = bm.halfEdges[hb ^ 1u];
         float sep = -FLT_MAX;
         Vector3 normal = Vector3::zero();
         if (gaussMapArcsCross(planes_a[a0.face].normal, planes_a[a1.face].normal,
@@ -1726,7 +1653,7 @@ __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &
         const bool face_contact_b = sep_b > e_sep;
         if (face_contact_a || face_contact_b) {
             const bool a_is_ref = sep_a >= sep_b;
-            const PPlane ref_plane = a_is_ref ? planes_a[face_a] : planes_b[face_b];
+            const Plane ref_plane = a_is_ref ? planes_a[face_a] : planes_b[face_b];
             const i32 ref_face = a_is_ref ? face_a : face_b;
             const HullInWorld &ref = a_is_ref ? a : b;
             const HullInWorld &inc = a_is_ref ? b : a;
@@ -1746,8 +1673,8 @@ __device__ bool hullHullGroup(EngineState &S, const PairSetup &ps, HullScratch &
         } else {
             // edge - edge: contact point on A's edge, depth = -separation, A is ref
             const u32 ha = ((u32)e_pair / eb) * 2, hb = ((u32)e_pair % eb) * 2;
-            const PHalfEdge he_a = am.halfEdges[ha];
-            const PHalfEdge he_b = bm.halfEdges[hb];
+            const HalfEdge he_a = am.halfEdges[ha];
+            const HalfEdge he_b = bm.halfEdges[hb];
             const Vector3 p = closestOnFirstSegment(
                 verts_a[he_a.rootVertex], verts_a[am.halfEdges[he_a.next].rootVertex],
                 verts_b[he_b.rootVertex], verts_b[bm.halfEdges[he_b.next].rootVertex]);
@@ -1811,7 +1738,7 @@ physNarrowSimpleKernel(EngineState *Sp)
             w = w0 + k;
             i = j - first[k];
             const size_t slot = (size_t)w * P.maxCandidatesPerWorld + i;
-            const PObjectManager &objs = worldObjects(S, P, w);
+            const ObjectManager &objs = worldObjects(S, P, w);
             const PairSetup ps = setupPair(S, P, objs, P.candidates[slot]);
             test = ps.test;
             bool hit = false;
@@ -1861,7 +1788,7 @@ physNarrowHullKernel(EngineState *Sp)
          e += (i32)gridDim.x * groups_per_block) {
         const HullQueueEntry ent = P.hullQueue[e];
         const size_t slot = (size_t)ent.world * P.maxCandidatesPerWorld + ent.cand;
-        const PObjectManager &objs = worldObjects(S, P, ent.world);
+        const ObjectManager &objs = worldObjects(S, P, ent.world);
         const PairSetup ps = setupPairImpl<false>(S, P, objs, P.candidates[slot]);
         const bool made = hullHullGroup(S, ps, scratch[group_in_block], gm, sub, P.contacts[slot]);
         if (sub == 0 && made) P.candHit[slot] = 1;
@@ -2011,8 +1938,8 @@ __device__ bool meanContact(const Contact &c, Vector3 *mean, float *deepest)
     return true;
 }
 
-__device__ __forceinline__ void localArms(const PPosRot &pre1, const PPosRot &pre2, Vector3 p1, float depth,
-                                          Vector3 n, Vector3 *r1, Vector3 *r2)
+__device__ __forceinline__ void localArms(const PreSolvePositional &pre1, const PreSolvePositional &pre2,
+                                          Vector3 p1, float depth, Vector3 n, Vector3 *r1, Vector3 *r2)
 {
     const Vector3 p2 = p1 - n * depth;
     *r1 = pre1.q.inv().rotateVec(p1 - pre1.x);
@@ -2020,27 +1947,27 @@ __device__ __forceinline__ void localArms(const PPosRot &pre1, const PPosRot &pr
 }
 
 __device__ __forceinline__ BodyPair bodyPair(const EngineState &S, const PhysicsState &P,
-                                             const PObjectManager &objs, u32 a1, i32 r1, u32 a2, i32 r2,
+                                             const ObjectManager &objs, u32 a1, i32 r1, u32 a2, i32 r2,
                                              float *mu_s, float *mu_d)
 {
-    const PMetadata m1 = objs.metadata[locCol<i32>(S, P, a1, r1, PCObjectID)];
-    const PMetadata m2 = objs.metadata[locCol<i32>(S, P, a2, r2, PCObjectID)];
-    BodyPair bp { m1.invMass, m2.invMass, m1.invInertia, m2.invInertia };
-    if (locCol<u32>(S, P, a1, r1, PCResponseType) == kRespStatic) {
+    const RigidBodyMetadata m1 = objs.metadata[locCol<i32>(S, P, a1, r1, PCObjectID)];
+    const RigidBodyMetadata m2 = objs.metadata[locCol<i32>(S, P, a2, r2, PCObjectID)];
+    BodyPair bp { m1.mass.invMass, m2.mass.invMass, m1.mass.invInertiaTensor, m2.mass.invInertiaTensor };
+    if (locCol<ResponseType>(S, P, a1, r1, PCResponseType) == ResponseType::Static) {
         bp.invM1 = 0.f;
         bp.invI1 = Vector3::zero();
     }
-    if (locCol<u32>(S, P, a2, r2, PCResponseType) == kRespStatic) {
+    if (locCol<ResponseType>(S, P, a2, r2, PCResponseType) == ResponseType::Static) {
         bp.invM2 = 0.f;
         bp.invI2 = Vector3::zero();
     }
-    *mu_s = 0.5f * (m1.muS + m2.muS);
-    *mu_d = 0.5f * (m1.muD + m2.muD);
+    *mu_s = 0.5f * (m1.friction.muS + m2.friction.muS);
+    *mu_d = 0.5f * (m1.friction.muD + m2.friction.muD);
     return bp;
 }
 
 // normal push-out along the contact normal + static friction (xpbd.cpp:347-419, 454-550)
-__device__ void solveContactPosition(EngineState &S, const PhysicsState &P, const PObjectManager &objs,
+__device__ void solveContactPosition(EngineState &S, const PhysicsState &P, const ObjectManager &objs,
                                      Contact &c)
 {
     c.lambdaN = 0.f;
@@ -2049,10 +1976,10 @@ __device__ void solveContactPosition(EngineState &S, const PhysicsState &P, cons
     Vector3 &x2_ref = locCol<Vector3>(S, P, c.altArch, c.altRow, PCPosition);
     Quat &q1_ref = locCol<Quat>(S, P, c.refArch, c.refRow, PCRotation);
     Quat &q2_ref = locCol<Quat>(S, P, c.altArch, c.altRow, PCRotation);
-    const PPosRot prev1 = locCol<PPosRot>(S, P, c.refArch, c.refRow, PCPrevState);
-    const PPosRot prev2 = locCol<PPosRot>(S, P, c.altArch, c.altRow, PCPrevState);
-    const PPosRot pre1 = locCol<PPosRot>(S, P, c.refArch, c.refRow, PCPreSolvePos);
-    const PPosRot pre2 = locCol<PPosRot>(S, P, c.altArch, c.altRow, PCPreSolvePos);
+    const SubstepPrevState prev1 = locCol<SubstepPrevState>(S, P, c.refArch, c.refRow, PCPrevState);
+    const SubstepPrevState prev2 = locCol<SubstepPrevState>(S, P, c.altArch, c.altRow, PCPrevState);
+    const PreSolvePositional pre1 = locCol<PreSolvePositional>(S, P, c.refArch, c.refRow, PCPreSolvePos);
+    const PreSolvePositional pre2 = locCol<PreSolvePositional>(S, P, c.altArch, c.altRow, PCPreSolvePos);
 
     float mu_s, mu_d;
     const BodyPair bp = bodyPair(S, P, objs, c.refArch, c.refRow, c.altArch, c.altRow, &mu_s, &mu_d);
@@ -2064,7 +1991,7 @@ __device__ void solveContactPosition(EngineState &S, const PhysicsState &P, cons
     float deepest;
     if (!meanContact(c, &mean, &deepest)) return;
 
-    const Vector3 n { c.normal.x, c.normal.y, c.normal.z };
+    const Vector3 n = c.normal;
     Vector3 r1, r2;
     localArms(pre1, pre2, mean, deepest, n, &r1, &r2);
 
@@ -2075,8 +2002,8 @@ __device__ void solveContactPosition(EngineState &S, const PhysicsState &P, cons
         const float lambda_n = positionalCorrection(x1, x2, q1, q2, r1, r2, bp, n, d, 0);
         c.lambdaN = lambda_n;
 
-        const Vector3 p1_hat = prev1.q.rotateVec(r1) + prev1.x;
-        const Vector3 p2_hat = prev2.q.rotateVec(r2) + prev2.x;
+        const Vector3 p1_hat = prev1.prevRotation.rotateVec(r1) + prev1.prevPosition;
+        const Vector3 p2_hat = prev2.prevRotation.rotateVec(r2) + prev2.prevPosition;
         p1 = q1.rotateVec(r1) + x1;
         p2 = q2.rotateVec(r2) + x2;
         const Vector3 dp = (p1 - p1_hat) - (p2 - p2_hat);
@@ -2120,13 +2047,13 @@ __device__ void angularCorrection(Quat &q1, Quat &q2, const BodyPair &bp, Vector
 }
 
 // fixed / hinge joints (xpbd.cpp:552-718)
-__device__ void solveJoint(EngineState &S, const PhysicsState &P, const PObjectManager &objs,
-                           const PJoint &j)
+__device__ void solveJoint(EngineState &S, const PhysicsState &P, const ObjectManager &objs,
+                           const JointConstraint &j)
 {
-    if (j.e1ID < 0 || j.e2ID < 0 || j.e1ID >= S.entityCapacity || j.e2ID >= S.entityCapacity) return;
-    const EntitySlot s1 = S.entitySlots[j.e1ID];
-    const EntitySlot s2 = S.entitySlots[j.e2ID];
-    if (s1.gen != j.e1Gen || s2.gen != j.e2Gen) return;
+    if (j.e1.id < 0 || j.e2.id < 0 || j.e1.id >= S.entityCapacity || j.e2.id >= S.entityCapacity) return;
+    const EntitySlot s1 = S.entitySlots[j.e1.id];
+    const EntitySlot s2 = S.entitySlots[j.e2.id];
+    if (s1.gen != j.e1.gen || s2.gen != j.e2.gen) return;
     const u32 a1 = (u32)s1.a, a2 = (u32)s2.a;
     const i32 r1row = s1.b, r2row = s2.b;
     if (!isBodyArchetype(a1) || !isBodyArchetype(a2)) return;
@@ -2142,7 +2069,7 @@ __device__ void solveJoint(EngineState &S, const PhysicsState &P, const PObjectM
     const BodyPair bp = bodyPair(S, P, objs, a1, r1row, a2, r2row, &mu_s, &mu_d);
 
     Vector3 correction;
-    if (j.type == 0) {
+    if (j.type == JointConstraint::Type::Fixed) {
         const Quat o1 = (q1 * j.fixed.attachRot1).normalize();
         const Quat o2 = (q2 * j.fixed.attachRot2).normalize();
         const Quat diff = o1 * o2.inv();
@@ -2249,7 +2176,7 @@ __device__ __forceinline__ void sweepContactLevels(const Contact *contacts, cons
 __device__ void phaseSolvePositions(EngineState &S, const PhysicsState &P, const i32 w, const bool valid,
                                     const int lane)
 {
-    const PObjectManager &objs = worldObjects(S, P, w);
+    const ObjectManager &objs = worldObjects(S, P, w);
 
     Contact *contacts = P.contacts + (size_t)w * P.maxCandidatesPerWorld;
     const i32 *order = P.contactOrder + (size_t)w * P.maxContactsPerWorld;
@@ -2261,7 +2188,7 @@ __device__ void phaseSolvePositions(EngineState &S, const PhysicsState &P, const
 
     const TableDesc &jt = S.tables[P.jointArchetype];
     if (valid && (lane & (kSolverLanes - 1)) == 0 && jt.numRows > 0) {
-        const PJoint *joints = (const PJoint *)jt.columns[P.jointCol];
+        const JointConstraint *joints = (const JointConstraint *)jt.columns[P.jointCol];
         const i32 *jw = (const i32 *)jt.columns[1];
         const i32 first = jt.worldOffsets[w];
         const i32 count = jt.worldCounts[w];
@@ -2280,24 +2207,24 @@ __device__ __forceinline__ Vector3 relativeVelocity(Vector3 v1, Vector3 v2, Vect
 
 // restitution on the mean contact, then dynamic friction per contact point
 // (xpbd.cpp:781-1039)
-__device__ void solveContactVelocity(EngineState &S, const PhysicsState &P, const PObjectManager &objs,
+__device__ void solveContactVelocity(EngineState &S, const PhysicsState &P, const ObjectManager &objs,
                                      const Contact &c, float h, float restitution_threshold)
 {
-    PVelocity &vel1_ref = locCol<PVelocity>(S, P, c.refArch, c.refRow, PCVelocity);
-    PVelocity &vel2_ref = locCol<PVelocity>(S, P, c.altArch, c.altRow, PCVelocity);
+    Velocity &vel1_ref = locCol<Velocity>(S, P, c.refArch, c.refRow, PCVelocity);
+    Velocity &vel2_ref = locCol<Velocity>(S, P, c.altArch, c.altRow, PCVelocity);
     const Quat q1 = locCol<Quat>(S, P, c.refArch, c.refRow, PCRotation);
     const Quat q2 = locCol<Quat>(S, P, c.altArch, c.altRow, PCRotation);
-    const PPosRot pre1 = locCol<PPosRot>(S, P, c.refArch, c.refRow, PCPreSolvePos);
-    const PPosRot pre2 = locCol<PPosRot>(S, P, c.altArch, c.altRow, PCPreSolvePos);
-    const PVelocity pv1 = locCol<PVelocity>(S, P, c.refArch, c.refRow, PCPreSolveVel);
-    const PVelocity pv2 = locCol<PVelocity>(S, P, c.altArch, c.altRow, PCPreSolveVel);
+    const PreSolvePositional pre1 = locCol<PreSolvePositional>(S, P, c.refArch, c.refRow, PCPreSolvePos);
+    const PreSolvePositional pre2 = locCol<PreSolvePositional>(S, P, c.altArch, c.altRow, PCPreSolvePos);
+    const PreSolveVelocity pv1 = locCol<PreSolveVelocity>(S, P, c.refArch, c.refRow, PCPreSolveVel);
+    const PreSolveVelocity pv2 = locCol<PreSolveVelocity>(S, P, c.altArch, c.altRow, PCPreSolveVel);
 
     float mu_s, mu_d;
     const BodyPair bp = bodyPair(S, P, objs, c.refArch, c.refRow, c.altArch, c.altRow, &mu_s, &mu_d);
 
     Vector3 v1 = vel1_ref.linear, o1 = vel1_ref.angular;
     Vector3 v2 = vel2_ref.linear, o2 = vel2_ref.angular;
-    const Vector3 n { c.normal.x, c.normal.y, c.normal.z };
+    const Vector3 n = c.normal;
 
     {
         Vector3 mean;
@@ -2306,7 +2233,7 @@ __device__ void solveContactVelocity(EngineState &S, const PhysicsState &P, cons
         Vector3 r1, r2;
         localArms(pre1, pre2, mean, deepest, n, &r1, &r2);
 
-        const Vector3 v_bar = relativeVelocity(pv1.linear, pv2.linear, pv1.angular, pv2.angular,
+        const Vector3 v_bar = relativeVelocity(pv1.v, pv2.v, pv1.omega, pv2.omega,
                                                pre1.q.rotateVec(r1), pre2.q.rotateVec(r2));
         const float vn_bar = dot(n, v_bar);
         const Vector3 r1_world = q1.rotateVec(r1);
@@ -2369,15 +2296,15 @@ __device__ void solveContactVelocity(EngineState &S, const PhysicsState &P, cons
         o2 -= q2.rotateVec(impulse * ra2);
     }
 
-    vel1_ref = PVelocity { v1, o1 };
-    vel2_ref = PVelocity { v2, o2 };
+    vel1_ref = Velocity { v1, o1 };
+    vel2_ref = Velocity { v2, o2 };
 }
 
 __device__ void phaseSolveVelocities(EngineState &S, const PhysicsState &P, const i32 w, const bool valid,
                                      const int lane)
 {
-    const PObjectManager &objs = worldObjects(S, P, w);
-    const PhysicsWorldParams &params = worldParams(S, P, w);
+    const ObjectManager &objs = worldObjects(S, P, w);
+    const PhysicsSystemState &params = worldParams(S, P, w);
     const Contact *contacts = P.contacts + (size_t)w * P.maxCandidatesPerWorld;
     const i32 *order = P.contactOrder + (size_t)w * P.maxContactsPerWorld;
     const i32 n = valid ? P.contactCounts[w] : 0;

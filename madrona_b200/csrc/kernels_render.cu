@@ -52,19 +52,14 @@ using madrona::math::Diag3x3;
 using madrona::math::AABB;
 using madrona::math::cross;
 using madrona::math::dot;
+using madrona::render::LightDesc;
+using madrona::render::RenderCamera;
 
 struct RenderHost {
     RenderState *dRender = nullptr;
     RenderState hRender;
     bool active = false;
     size_t tlasSmem = 0;
-};
-
-struct RenderCameraComp {     // == madrona::render::RenderCamera
-    u32 outGen; i32 outID;
-    float fovScale;
-    float zNear;
-    Vector3 cameraOffset;
 };
 
 // ---- render-prepare: instances ---------------------------------------------------------
@@ -99,9 +94,9 @@ renderGatherInstancesKernel(EngineState *Sp)
                     const Vector3 p = ((const Vector3 *)t.columns[ra.cols[RCPosition]])[row];
                     const Quat q = ((const Quat *)t.columns[ra.cols[RCRotation]])[row];
                     const Diag3x3 s = ((const Diag3x3 *)t.columns[ra.cols[RCScale]])[row];
-                    inst.position = RVec3 { p.x, p.y, p.z };
-                    inst.rotation = RQuat { q.w, q.x, q.y, q.z };
-                    inst.scale = RVec3 { s.d0, s.d1, s.d2 };
+                    inst.position = p;
+                    inst.rotation = q;
+                    inst.scale = Vector3 { s.d0, s.d1, s.d2 };
                     inst.objectID = ((const i32 *)t.columns[ra.cols[RCObjectID]])[row];
                     // instanceTransformUpdate (no material components: mesh default) /
                     // instanceTransformUpdateWithMat (ecs_system.cpp:100-159, 211-250); a
@@ -152,16 +147,16 @@ renderLightUpdateKernel(EngineState *Sp, u32 archetype, i32 carrier_col, i32 pos
         if (id < 0 || id >= S.entityCapacity) continue;
         const EntitySlot slot = S.entitySlots[id];
         if (slot.gen != gen || (u32)slot.a != R.lightArchetype) continue;
-        LightDescComp &d = ((LightDescComp *)S.tables[R.lightArchetype].columns[R.lightCol])[slot.b];
+        LightDesc &d = ((LightDesc *)S.tables[R.lightArchetype].columns[R.lightCol])[slot.b];
         const Vector3 p = ((const Vector3 *)t.columns[pos_col])[row];
         const Vector3 dir = ((const Vector3 *)t.columns[dir_col])[row];
-        d.type = ((const unsigned char *)t.columns[type_col])[row];
-        d.castShadow = ((const unsigned char *)t.columns[shadow_col])[row];
-        d.position[0] = p.x; d.position[1] = p.y; d.position[2] = p.z;
-        d.direction[0] = dir.x; d.direction[1] = dir.y; d.direction[2] = dir.z;
+        d.type = ((const LightDesc::Type *)t.columns[type_col])[row];
+        d.castShadow = ((const bool *)t.columns[shadow_col])[row];
+        d.position = p;
+        d.direction = dir;
         d.cutoff = ((const float *)t.columns[cutoff_col])[row];
         d.intensity = ((const float *)t.columns[intensity_col])[row];
-        d.active = ((const unsigned char *)t.columns[active_col])[row];
+        d.active = ((const bool *)t.columns[active_col])[row];
     }
 }
 
@@ -178,12 +173,12 @@ renderGatherLightsKernel(EngineState *Sp)
         i32 kept = 0;
         for (i32 r = first; r < first + count && kept < kMaxLightsPerWorld; r++) {
             if (((const i32 *)t.columns[1])[r] != w) continue;
-            const LightDescComp d = ((const LightDescComp *)t.columns[R.lightCol])[r];
+            const LightDesc d = ((const LightDesc *)t.columns[R.lightCol])[r];
             RenderLight l;
             l.directional = d.type ? 1u : 0u;
             l.castShadow = d.castShadow ? 1u : 0u;
-            l.position = RVec3 { d.position[0], d.position[1], d.position[2] };
-            l.direction = RVec3 { d.direction[0], d.direction[1], d.direction[2] };
+            l.position = d.position;
+            l.direction = d.direction;
             l.cutoff = d.cutoff;
             l.intensity = d.intensity;
             l.active = d.active ? 1u : 0u;
@@ -211,10 +206,11 @@ renderGatherViewsKernel(EngineState *Sp)
     for (i32 row = blockIdx.x * blockDim.x + threadIdx.x; row < n; row += gridDim.x * blockDim.x) {
         const i32 w = world_col[row];
         if (w < 0) continue;
-        const RenderCameraComp cam = ((const RenderCameraComp *)t.columns[va.camCol])[row];
-        if (cam.outID < 0 || cam.outID >= S.entityCapacity) continue;
-        const EntitySlot slot = S.entitySlots[cam.outID];
-        if (slot.gen != cam.outGen || (u32)slot.a != R.outputArchetype) continue;
+        const RenderCamera cam = ((const RenderCamera *)t.columns[va.camCol])[row];
+        const madrona::Entity out = cam.cameraEntity;
+        if (out.id < 0 || out.id >= S.entityCapacity) continue;
+        const EntitySlot slot = S.entitySlots[out.id];
+        if (slot.gen != out.gen || (u32)slot.a != R.outputArchetype) continue;
         const i32 out_row = slot.b;
         if (out_row < 0 || out_row >= R.maxViews) continue;
         const Vector3 p = ((const Vector3 *)t.columns[va.posCol])[row];
@@ -222,8 +218,8 @@ renderGatherViewsKernel(EngineState *Sp)
         const Vector3 cam_pos = p + cam.cameraOffset;
         const Quat inv = q.inv();
         RenderView v;
-        v.position = RVec3 { cam_pos.x, cam_pos.y, cam_pos.z };
-        v.rotation = RQuat { inv.w, inv.x, inv.y, inv.z };
+        v.position = cam_pos;
+        v.rotation = inv;
         v.xScale = cam.fovScale;          // square output: aspect ratio 1
         v.yScale = -cam.fovScale;
         v.zNear = cam.zNear;
@@ -749,7 +745,7 @@ __device__ RayHit traceWorld(const RenderState &R, const QBVHNode *tlas, const i
             const RenderInstance &inst = instances[ii];
             if (!instanceTraceable(R, inst)) continue;
             const InstanceXform X = instanceXform(inst);
-            const Vector3 oo = applyLinear(X.m, o - Vector3 { inst.position.x, inst.position.y, inst.position.z });
+            const Vector3 oo = applyLinear(X.m, o - inst.position);
             const Vector3 od = applyLinear(X.m, d);
             int tri = -1;
             if (traceMesh<ANY_HIT>(R.meshes[inst.objectID], oo, od, t_min, hit.t, tri, stack, sp)) {
@@ -873,8 +869,8 @@ renderRaycastKernel(EngineState *Sp)
         if ((num_instances <= kFlatInstances) != FLAT) continue;
 
         // camera frame (shared by every pixel of the view)
-        const Quat rot { view.rotation.w, view.rotation.x, view.rotation.y, view.rotation.z };
-        const Vector3 ray_start { view.position.x, view.position.y, view.position.z };
+        const Quat rot = view.rotation;
+        const Vector3 ray_start = view.position;
         const Vector3 look_at = rot.inv().rotateVec({ 0, 1, 0 });
         const float h = 1.0f / (-view.yScale);
         const float viewport = 2 * h;
@@ -895,8 +891,7 @@ renderRaycastKernel(EngineState *Sp)
 #pragma unroll
                 for (int k = 0; k < 9; k++) fi.m[k] = X.m[k];
                 fi.pos[0] = inst.position.x; fi.pos[1] = inst.position.y; fi.pos[2] = inst.position.z;
-                const Vector3 oo = applyLinear(X.m, ray_start - Vector3 { inst.position.x, inst.position.y,
-                                                                           inst.position.z });
+                const Vector3 oo = applyLinear(X.m, ray_start - inst.position);
                 fi.oo[0] = oo.x; fi.oo[1] = oo.y; fi.oo[2] = oo.z;
                 float lo[3], hi[3];
                 float dist2 = 0.f;
@@ -1028,17 +1023,17 @@ renderRaycastKernel(EngineState *Sp)
                     const Vector3 ta { tv[0].pos[0], tv[0].pos[1], tv[0].pos[2] };
                     const Vector3 tb { tv[1].pos[0], tv[1].pos[1], tv[1].pos[2] };
                     const Vector3 tc { tv[2].pos[0], tv[2].pos[1], tv[2].pos[2] };
-                    const Quat iq { inst.rotation.w, inst.rotation.x, inst.rotation.y, inst.rotation.z };
+                    const Quat iq = inst.rotation;
                     const Vector3 normal = iq.rotateVec(madrona::math::normalize(cross(tb - ta, tc - ta)));
 
                     // lights (bvh_raycast.cpp:861-919)
                     const Vector3 hit_pos = ray_start + first.t * ray_dir;
                     for (i32 li = 0; li < num_lights; li++) {
                         const RenderLight &l = lights[li];
-                        const Vector3 ldir_in { l.direction.x, l.direction.y, l.direction.z };
+                        const Vector3 ldir_in = l.direction;
                         Vector3 light_dir = -ldir_in;
                         if (!l.directional) {
-                            light_dir = (Vector3 { l.position.x, l.position.y, l.position.z } - hit_pos).normalize();
+                            light_dir = (l.position - hit_pos).normalize();
                             if (l.cutoff != -1.f) {
                                 float dd = dot(-light_dir, ldir_in);
                                 dd /= (light_dir.length() * ldir_in.length());

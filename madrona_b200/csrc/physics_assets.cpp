@@ -16,8 +16,7 @@
 // (build_convex_hulls = true) is not provided.
 #include "../../include/madrona_b200.h"
 #include "engine.hpp"
-
-#include <madrona/math.hpp>
+#include "physics_state.h"
 
 #include <cfloat>
 #include <cstring>
@@ -32,53 +31,24 @@ using madrona::math::Diag3x3;
 using madrona::math::Mat3x3;
 using madrona::math::Symmetric3x3;
 using madrona::math::AABB;
+using madrona::geo::HalfEdge;
+using madrona::geo::HalfEdgeMesh;
+using madrona::geo::Plane;
+using madrona::phys::CollisionPrimitive;
+using madrona::phys::ObjectManager;
+using madrona::phys::RigidBodyMetadata;
 
 namespace {
 
-// == geo::HalfEdge / geo::Plane / geo::HalfEdgeMesh / phys::CollisionPrimitive /
-// RigidBodyMetadata / ObjectManager (include/madrona/geo.hpp:7-45, physics.hpp:84-153)
-struct AHalfEdge { uint32_t next, rootVertex, face; };
-struct APlane { Vector3 normal; float d; };
-struct AHalfEdgeMesh {
-    AHalfEdge *halfEdges;
-    uint32_t *faceBaseHalfEdges;
-    APlane *facePlanes;
-    Vector3 *vertices;
-    uint32_t numHalfEdges, numFaces, numVertices;
-};
-struct APrimitive {
-    uint32_t type;
-    union {
-        float sphereRadius;
-        AHalfEdgeMesh hull;
-    };
-};
-struct AMetadata {
-    float invMass;
-    Vector3 invInertiaTensor;
-    Vector3 toCenterOfMass;
-    Quat toInertiaFrame;
-    float muS, muD;
-};
-struct AObjectManager {
-    APrimitive *collisionPrimitives;
-    AABB *primitiveAABBs;
-    AABB *rigidBodyAABBs;
-    uint32_t *rigidBodyPrimitiveOffsets;
-    uint32_t *rigidBodyPrimitiveCounts;
-    AMetadata *metadata;
-};
-static_assert(sizeof(APrimitive) == 56 && sizeof(AMetadata) == 52 && sizeof(AObjectManager) == 48, "layouts");
-
 struct HostHull {
-    std::vector<AHalfEdge> hedges;
+    std::vector<HalfEdge> hedges;
     std::vector<uint32_t> faceBase;
-    std::vector<APlane> planes;
+    std::vector<Plane> planes;
     std::vector<Vector3> verts;
 };
 
 // RTCD 12.4.2 (physics_assets.cpp:211-252): normal from the projected areas, d through the centroid
-APlane newellPlane(const Vector3 *verts, const uint32_t *indices, int64_t n)
+Plane newellPlane(const Vector3 *verts, const uint32_t *indices, int64_t n)
 {
     Vector3 centroid { 0, 0, 0 };
     Vector3 nrm { 0, 0, 0 };
@@ -94,7 +64,7 @@ APlane newellPlane(const Vector3 *verts, const uint32_t *indices, int64_t n)
     }
     centroid /= (float)count;
     nrm = madrona::math::normalize(nrm);
-    return APlane { nrm, madrona::math::dot(centroid, nrm) };
+    return Plane { nrm, madrona::math::dot(centroid, nrm) };
 }
 
 // buildHalfEdgeMesh (physics_assets.cpp:638-748): an edge gets the next two half-edge
@@ -111,7 +81,7 @@ bool buildHull(const mb2_source_hull &src, HostHull *out, std::string *err)
     }
     out->verts.resize(src.num_vertices);
     memcpy(out->verts.data(), src.positions, sizeof(Vector3) * src.num_vertices);
-    out->hedges.assign(num_hedges, AHalfEdge { 0, 0, 0 });
+    out->hedges.assign(num_hedges, HalfEdge { 0, 0, 0 });
     out->faceBase.resize(src.num_faces);
     out->planes.resize(src.num_faces);
 
@@ -144,7 +114,7 @@ bool buildHull(const mb2_source_hull &src, HostHull *out, std::string *err)
             if (k == 0) out->faceBase[f] = hedge;
             auto next_it = edge_to_hedge.find(edge_id(b, c));
             const uint32_t next = next_it == edge_to_hedge.end() ? assigned : next_it->second;
-            out->hedges[hedge] = AHalfEdge { next, a, f };
+            out->hedges[hedge] = HalfEdge { next, a, f };
         }
         idx += nv;
     }
@@ -284,14 +254,14 @@ MassProps massProperties(const std::vector<HostHull> &hulls, const mb2_source_ob
         const HostHull &h = hulls[prim.hull_idx];
         for (size_t f = 0; f < h.faceBase.size(); f++) {
             const uint32_t root_idx = h.faceBase[f];
-            const AHalfEdge root = h.hedges[root_idx];
+            const HalfEdge root = h.hedges[root_idx];
             const Vector3 v1 = h.verts[root.rootVertex];
             uint32_t cur_idx = root.next;
             while (true) {
-                const AHalfEdge cur = h.hedges[cur_idx];
+                const HalfEdge cur = h.hedges[cur_idx];
                 const uint32_t next_idx = cur.next;
                 if (next_idx == root_idx) break;
-                const AHalfEdge next = h.hedges[next_idx];
+                const HalfEdge next = h.hedges[next_idx];
                 tet(v1, h.verts[cur.rootVertex], h.verts[next.rootVertex]);
                 cur_idx = next_idx;
             }
@@ -339,7 +309,7 @@ Layout layoutFor(const size_t sizes[10])
 struct ObjectManagerBundle {
     int gpu = -1;
     std::vector<char> hostBlob;        // arrays, pointers valid on the host
-    AObjectManager hostMgr {};
+    ObjectManager hostMgr {};
     void *deviceBlob = nullptr;        // arrays + the ObjectManager struct at the end
     void *deviceMgr = nullptr;
     mb2_rigid_body_assets view {};
@@ -386,37 +356,37 @@ mb2_object_manager *mb2_process_rigid_body_assets(const mb2_source_hull *hulls, 
     // same buffer order as the reference: halfEdges, faceBaseHalfEdges, facePlanes, vertices,
     // primitives, primitiveAABBs, metadatas, objAABBs, primOffsets, primCounts
     const size_t sizes[10] = {
-        sizeof(AHalfEdge) * n_he, sizeof(uint32_t) * n_faces, sizeof(APlane) * n_faces, sizeof(Vector3) * n_verts,
-        sizeof(APrimitive) * n_prims, sizeof(AABB) * n_prims, sizeof(AMetadata) * num_objects,
+        sizeof(HalfEdge) * n_he, sizeof(uint32_t) * n_faces, sizeof(Plane) * n_faces, sizeof(Vector3) * n_verts,
+        sizeof(CollisionPrimitive) * n_prims, sizeof(AABB) * n_prims, sizeof(RigidBodyMetadata) * num_objects,
         sizeof(AABB) * num_objects, sizeof(uint32_t) * num_objects, sizeof(uint32_t) * num_objects,
     };
     const Layout L = layoutFor(sizes);
     ObjectManagerBundle *b = new ObjectManagerBundle();
     b->gpu = gpu_id;
-    b->hostBlob.assign(L.total + sizeof(AObjectManager), 0);
+    b->hostBlob.assign(L.total + sizeof(ObjectManager), 0);
     char *base = b->hostBlob.data();
-    AHalfEdge *he_out = (AHalfEdge *)(base + L.offsets[0]);
+    HalfEdge *he_out = (HalfEdge *)(base + L.offsets[0]);
     uint32_t *fb_out = (uint32_t *)(base + L.offsets[1]);
-    APlane *pl_out = (APlane *)(base + L.offsets[2]);
+    Plane *pl_out = (Plane *)(base + L.offsets[2]);
     Vector3 *vt_out = (Vector3 *)(base + L.offsets[3]);
-    APrimitive *prims = (APrimitive *)(base + L.offsets[4]);
+    CollisionPrimitive *prims = (CollisionPrimitive *)(base + L.offsets[4]);
     AABB *prim_aabbs = (AABB *)(base + L.offsets[5]);
-    AMetadata *metas = (AMetadata *)(base + L.offsets[6]);
+    RigidBodyMetadata *metas = (RigidBodyMetadata *)(base + L.offsets[6]);
     AABB *obj_aabbs = (AABB *)(base + L.offsets[7]);
     uint32_t *prim_offsets = (uint32_t *)(base + L.offsets[8]);
     uint32_t *prim_counts = (uint32_t *)(base + L.offsets[9]);
 
-    std::vector<AHalfEdgeMesh> meshes(num_hulls);
+    std::vector<HalfEdgeMesh> meshes(num_hulls);
     size_t he_at = 0, f_at = 0, v_at = 0;
     for (uint32_t h = 0; h < num_hulls; h++) {
         const HostHull &hh = built[h];
-        memcpy(he_out + he_at, hh.hedges.data(), sizeof(AHalfEdge) * hh.hedges.size());
+        memcpy(he_out + he_at, hh.hedges.data(), sizeof(HalfEdge) * hh.hedges.size());
         memcpy(fb_out + f_at, hh.faceBase.data(), sizeof(uint32_t) * hh.faceBase.size());
-        memcpy(pl_out + f_at, hh.planes.data(), sizeof(APlane) * hh.planes.size());
+        memcpy(pl_out + f_at, hh.planes.data(), sizeof(Plane) * hh.planes.size());
         memcpy(vt_out + v_at, hh.verts.data(), sizeof(Vector3) * hh.verts.size());
-        meshes[h] = AHalfEdgeMesh { he_out + he_at, fb_out + f_at, pl_out + f_at, vt_out + v_at,
-                                    (uint32_t)hh.hedges.size(), (uint32_t)hh.faceBase.size(),
-                                    (uint32_t)hh.verts.size() };
+        meshes[h] = HalfEdgeMesh { he_out + he_at, fb_out + f_at, pl_out + f_at, vt_out + v_at,
+                                   (uint32_t)hh.hedges.size(), (uint32_t)hh.faceBase.size(),
+                                   (uint32_t)hh.verts.size() };
         he_at += hh.hedges.size();
         f_at += hh.faceBase.size();
         v_at += hh.verts.size();
@@ -428,21 +398,21 @@ mb2_object_manager *mb2_process_rigid_body_assets(const mb2_source_hull *hulls, 
         AABB obj_box = AABB::invalid();
         for (uint32_t p = 0; p < objects[o].num_prims; p++) {
             const mb2_source_prim &src = objects[o].prims[p];
-            APrimitive &out = prims[prim_at + p];
+            CollisionPrimitive &out = prims[prim_at + p];
             memset(&out, 0, sizeof(out));
-            out.type = src.type;
+            out.type = (CollisionPrimitive::Type)src.type;
             AABB box;
             if (src.type == 1) {
-                out.sphereRadius = src.sphere_radius;
+                out.sphere.radius = src.sphere_radius;
                 const float r = src.sphere_radius;
                 box = AABB { { -r, -r, -r }, { r, r, r } };
             } else if (src.type == 4) {
                 box = AABB { { -FLT_MAX, -FLT_MAX, -FLT_MAX }, { FLT_MAX, FLT_MAX, 0 } };
             } else {
-                const AHalfEdgeMesh &m = meshes[src.hull_idx];
+                const HalfEdgeMesh &m = meshes[src.hull_idx];
                 box = AABB::point(m.vertices[0]);
                 for (uint32_t v = 1; v < m.numVertices; v++) box.expand(m.vertices[v]);
-                out.hull = m;
+                out.hull.halfEdgeMesh = m;
             }
             prim_aabbs[prim_at + p] = box;
             obj_box = AABB::merge(obj_box, box);
@@ -456,14 +426,16 @@ mb2_object_manager *mb2_process_rigid_body_assets(const mb2_source_hull *hulls, 
     for (uint32_t o = 0; o < num_objects; o++) {
         const MassProps mp = massProperties(built, objects[o]);
         const Diag3x3 inv_inertia = objects[o].inv_mass / mp.inertia;
-        metas[o] = AMetadata { objects[o].inv_mass, Vector3 { inv_inertia.d0, inv_inertia.d1, inv_inertia.d2 },
-                               mp.com, mp.toDiagonal, objects[o].mu_s, objects[o].mu_d };
+        metas[o] = RigidBodyMetadata {
+            { objects[o].inv_mass, Vector3 { inv_inertia.d0, inv_inertia.d1, inv_inertia.d2 }, mp.com, mp.toDiagonal },
+            { objects[o].mu_s, objects[o].mu_d },
+        };
     }
     b->view = mb2_rigid_body_assets { he_out, fb_out, pl_out, vt_out, (uint32_t)n_he, (uint32_t)n_faces,
                                       (uint32_t)n_verts, prims, prim_aabbs, metas, obj_aabbs, prim_offsets,
                                       prim_counts, num_hulls, (uint32_t)n_prims, num_objects };
-    b->hostMgr = AObjectManager { prims, prim_aabbs, obj_aabbs, prim_offsets, prim_counts, metas };
-    memcpy(base + L.total, &b->hostMgr, sizeof(AObjectManager));
+    b->hostMgr = ObjectManager { prims, prim_aabbs, obj_aabbs, prim_offsets, prim_counts, metas };
+    memcpy(base + L.total, &b->hostMgr, sizeof(ObjectManager));
 
     if (gpu_id >= 0) {
         // PhysicsLoader::loadRigidBodies: the same block on the GPU, pointers rebased
@@ -476,22 +448,23 @@ mb2_object_manager *mb2_process_rigid_body_assets(const mb2_source_hull *hulls, 
         std::vector<char> staged = b->hostBlob;
         const ptrdiff_t delta = (char *)b->deviceBlob - base;
         auto rebase = [&](void *p) { return p ? (void *)((char *)p + delta) : nullptr; };
-        APrimitive *sp = (APrimitive *)(staged.data() + L.offsets[4]);
+        CollisionPrimitive *sp = (CollisionPrimitive *)(staged.data() + L.offsets[4]);
         for (size_t i = 0; i < n_prims; i++) {
-            if (sp[i].type == 2) {
-                sp[i].hull.halfEdges = (AHalfEdge *)rebase(sp[i].hull.halfEdges);
-                sp[i].hull.faceBaseHalfEdges = (uint32_t *)rebase(sp[i].hull.faceBaseHalfEdges);
-                sp[i].hull.facePlanes = (APlane *)rebase(sp[i].hull.facePlanes);
-                sp[i].hull.vertices = (Vector3 *)rebase(sp[i].hull.vertices);
+            if (sp[i].type == CollisionPrimitive::Type::Hull) {
+                HalfEdgeMesh &m = sp[i].hull.halfEdgeMesh;
+                m.halfEdges = (HalfEdge *)rebase(m.halfEdges);
+                m.faceBaseHalfEdges = (uint32_t *)rebase(m.faceBaseHalfEdges);
+                m.facePlanes = (Plane *)rebase(m.facePlanes);
+                m.vertices = (Vector3 *)rebase(m.vertices);
             }
         }
-        AObjectManager dm = b->hostMgr;
-        dm.collisionPrimitives = (APrimitive *)rebase(dm.collisionPrimitives);
+        ObjectManager dm = b->hostMgr;
+        dm.collisionPrimitives = (CollisionPrimitive *)rebase(dm.collisionPrimitives);
         dm.primitiveAABBs = (AABB *)rebase(dm.primitiveAABBs);
         dm.rigidBodyAABBs = (AABB *)rebase(dm.rigidBodyAABBs);
         dm.rigidBodyPrimitiveOffsets = (uint32_t *)rebase(dm.rigidBodyPrimitiveOffsets);
         dm.rigidBodyPrimitiveCounts = (uint32_t *)rebase(dm.rigidBodyPrimitiveCounts);
-        dm.metadata = (AMetadata *)rebase(dm.metadata);
+        dm.metadata = (RigidBodyMetadata *)rebase(dm.metadata);
         memcpy(staged.data() + L.total, &dm, sizeof(dm));
         cudaMemcpy(b->deviceBlob, staged.data(), staged.size(), cudaMemcpyHostToDevice);
         b->deviceMgr = (char *)b->deviceBlob + L.total;
@@ -503,7 +476,7 @@ void *mb2_object_manager_ptr(const mb2_object_manager *mgr, int device)
 {
     const ObjectManagerBundle *b = (const ObjectManagerBundle *)mgr;
     if (!b) return nullptr;
-    return device ? b->deviceMgr : (void *)(b->hostBlob.data() + b->hostBlob.size() - sizeof(AObjectManager));
+    return device ? b->deviceMgr : (void *)(b->hostBlob.data() + b->hostBlob.size() - sizeof(ObjectManager));
 }
 
 void mb2_object_manager_host_assets(const mb2_object_manager *mgr, mb2_rigid_body_assets *out)

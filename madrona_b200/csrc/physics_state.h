@@ -1,6 +1,8 @@
 // physics_state.h -- layouts shared by the NVRTC-side physics API
-// (device/madrona/physics.hpp: what simulator code calls) and the ahead-of-time
-// physics kernels (kernels_physics.cu).  Plain structs, no std headers.
+// (device/madrona/physics.hpp: what simulator code calls), the ahead-of-time
+// physics kernels (kernels_physics.cu) and the host asset builder
+// (physics_assets.cpp).  Plain structs; every header included here compiles
+// under g++, nvcc and NVRTC.
 //
 // The public component structs (Velocity, CollisionPrimitive, ObjectManager,
 // RigidBodyMetadata, HalfEdgeMesh ...) keep the reference's field order and
@@ -10,14 +12,165 @@
 // BVH storage) is laid out for the GPU instead of being ECS archetypes.
 #pragma once
 
+#include <cstddef>
+#include <madrona/math.hpp>
+#include <madrona/geo.hpp>
+#include <madrona/ecs.hpp>
+
 #include "mb2_state.h"
+
+namespace madrona::phys {
+
+enum class ResponseType : uint32_t {
+    Dynamic,
+    Kinematic,
+    Static,
+};
+
+struct Velocity {
+    math::Vector3 linear;
+    math::Vector3 angular;
+};
+
+struct JointConstraint {
+    enum class Type {
+        Fixed,
+        Hinge
+    };
+
+    struct Fixed {
+        math::Quat attachRot1;
+        math::Quat attachRot2;
+        float separation;
+    };
+
+    struct Hinge {
+        math::Vector3 a1Local;
+        math::Vector3 a2Local;
+        math::Vector3 b1Local;
+        math::Vector3 b2Local;
+    };
+
+    Entity e1;
+    Entity e2;
+    Type type;
+
+    union {
+        Fixed fixed;
+        Hinge hinge;
+    };
+
+    math::Vector3 r1;
+    math::Vector3 r2;
+};
+
+struct RigidBodyMassData {
+    float invMass;
+    math::Vector3 invInertiaTensor;
+    math::Vector3 toCenterOfMass;
+    math::Quat toInteriaFrame;
+};
+
+struct RigidBodyFrictionData {
+    float muS;
+    float muD;
+};
+
+struct RigidBodyMetadata {
+    RigidBodyMassData mass;
+    RigidBodyFrictionData friction;
+};
+
+struct CollisionPrimitive {
+    enum class Type : uint32_t {
+        Sphere = 1 << 0,
+        Hull = 1 << 1,
+        Plane = 1 << 2,
+    };
+
+    struct Sphere {
+        float radius;
+    };
+
+    struct Hull {
+        geo::HalfEdgeMesh halfEdgeMesh;
+    };
+
+    struct Plane {};
+
+    Type type;
+    union {
+        Sphere sphere;
+        Plane plane;
+        Hull hull;
+    };
+};
+
+struct ObjectManager {
+    CollisionPrimitive *collisionPrimitives;
+    math::AABB *primitiveAABBs;
+
+    math::AABB *rigidBodyAABBs;
+    uint32_t *rigidBodyPrimitiveOffsets;
+    uint32_t *rigidBodyPrimitiveCounts;
+    RigidBodyMetadata *metadata;
+};
+
+// == src/physics/physics_impl.hpp:7-15 (a singleton component, per world)
+struct PhysicsSystemState {
+    float deltaT;
+    float h;
+    math::Vector3 g;
+    float gMagnitude;
+    float restitutionThreshold;
+    uint32_t contactArchetypeID;
+    uint32_t jointArchetypeID;
+};
+
+namespace xpbd {
+
+// == src/physics/xpbd.cpp:26-46
+struct SubstepPrevState {
+    math::Vector3 prevPosition;
+    math::Quat prevRotation;
+};
+
+struct PreSolvePositional {
+    math::Vector3 x;
+    math::Quat q;
+};
+
+struct PreSolveVelocity {
+    math::Vector3 v;
+    math::Vector3 omega;
+};
+
+}
+
+// The kernels read these through ECS columns and the uploaded ObjectManager blob,
+// and RigidBodyAssets.host_arrays (executor.py) decodes the blob by offset.
+static_assert(sizeof(Velocity) == 24, "Velocity layout");
+static_assert(sizeof(JointConstraint) == 92, "JointConstraint layout");
+static_assert(sizeof(RigidBodyMetadata) == 52, "RigidBodyMetadata layout");
+static_assert(sizeof(CollisionPrimitive) == 56, "CollisionPrimitive layout");
+static_assert(sizeof(ObjectManager) == 48, "ObjectManager layout");
+static_assert(sizeof(PhysicsSystemState) == 36, "PhysicsSystemState layout");
+static_assert(sizeof(geo::HalfEdge) == 12 && sizeof(geo::Plane) == 16 && sizeof(math::AABB) == 24,
+              "object description element layouts");
+#ifndef __CUDACC_RTC__    // NVRTC has no constant offsetof
+static_assert(offsetof(CollisionPrimitive, sphere) == 8 && offsetof(CollisionPrimitive, hull) == 8,
+              "CollisionPrimitive layout");
+static_assert(offsetof(geo::HalfEdgeMesh, halfEdges) == 0 && offsetof(geo::HalfEdgeMesh, faceBaseHalfEdges) == 8 &&
+              offsetof(geo::HalfEdgeMesh, facePlanes) == 16 && offsetof(geo::HalfEdgeMesh, vertices) == 24 &&
+              offsetof(geo::HalfEdgeMesh, numHalfEdges) == 32 && offsetof(geo::HalfEdgeMesh, numFaces) == 36 &&
+              offsetof(geo::HalfEdgeMesh, numVertices) == 40, "HalfEdgeMesh layout");
+#endif
+
+}
 
 namespace mb2 {
 
-struct PVec3 { float x, y, z; };
-struct PQuat { float w, x, y, z; };
 struct alignas(16) PVec4 { float x, y, z, w; };
-struct PAABB { PVec3 pMin, pMax; };
 
 // == broadphase::BVH::Node (include/madrona/broadphase.hpp:62-78): 4-wide node,
 // child boxes in SoA, leaf children tagged with bit 31, sentinel = -1.
@@ -31,20 +184,21 @@ struct BVHNode {
     i32 children[4];
     i32 parentID;
 };
+static_assert(sizeof(BVHNode) == 116, "BVH node layout");
 
 struct LeafTransform {
-    PVec3 pos;
-    PQuat rot;
-    PVec3 scale;
+    madrona::math::Vector3 pos;
+    madrona::math::Quat rot;
+    madrona::math::Vector3 scale;
 };
 
 // One per world: the payload of the broadphase::BVH singleton component.
 struct WorldBVH {
     BVHNode *nodes;
     u64 *leafEntities;        // Entity {gen,id} packed as in the table column
-    const void *objMgr;       // const phys::ObjectManager *
+    const madrona::phys::ObjectManager *objMgr;
     i32 *leafObjIDs;
-    PAABB *leafAABBs;
+    madrona::math::AABB *leafAABBs;
     LeafTransform *leafTransforms;
     u32 *leafParents;         // (node << 2) | child
     i32 *sortedLeaves;
@@ -70,17 +224,6 @@ struct WorldBVH {
     i32 numTraversal;
 };
 
-// == phys::PhysicsSystemState (src/physics/physics_impl.hpp:7-15)
-struct PhysicsWorldParams {
-    float deltaT;
-    float h;
-    PVec3 g;
-    float gMagnitude;
-    float restitutionThreshold;
-    u32 contactArchetypeID;
-    u32 jointArchetypeID;
-};
-
 // Role of phys::CandidateCollision (physics.hpp:52-57: two Locs + two primitive
 // indices, 24 B), packed to 16 B and extended with what the narrowphase would
 // otherwise look up again per contact:
@@ -95,6 +238,7 @@ struct Candidate {
     i32 bRow;
     u32 slots;
 };
+static_assert(sizeof(Candidate) == 16, "candidate layout");
 
 struct HullQueueEntry {
     i32 world;
@@ -107,7 +251,7 @@ struct Contact {
     u32 altArch; i32 altRow;
     float points[4][4];       // xyz + penetration depth
     i32 numPoints;
-    PVec3 normal;
+    madrona::math::Vector3 normal;
     float lambdaN;            // XPBDContactState::lambdaN[0], the only one ever read (xpbd.cpp:1028)
     u32 refInfo;              // (world body slot << 1) | mutable of ref / alt (Candidate::slots)
     u32 altInfo;
@@ -117,6 +261,7 @@ struct Contact {
     // bit-identical to the reference's sequential Gauss-Seidel sweep.
     i32 level;
 };
+static_assert(sizeof(Contact) == 112, "contact layout");
 
 enum PhysCol : int {
     PCPosition = 0, PCRotation, PCScale, PCObjectID, PCResponseType, PCLeafID,

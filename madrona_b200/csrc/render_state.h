@@ -3,20 +3,49 @@
 // (kernels_render.cu).  SURVEY.md 8 rows a13-a15.
 #pragma once
 
+#include <madrona/math.hpp>
+#include <madrona/ecs.hpp>
+
 #include "mb2_state.h"
 #include "render_bvh.h"
 
-namespace mb2 {
+namespace madrona::render {
 
-struct RVec3 { float x, y, z; };
-struct RQuat { float w, x, y, z; };
+struct RenderCamera {
+    Entity cameraEntity;      // the view's RaycastOutputArchetype entity
+    float fovScale;
+    float zNear;
+    math::Vector3 cameraOffset;
+};
+
+// == include/madrona/render/ecs.hpp:65-115
+struct LightDesc {
+    enum Type : bool {
+        Directional = true,
+        Spotlight = false
+    };
+    Type type;
+    bool castShadow;
+    math::Vector3 position;
+    math::Vector3 direction;
+    float cutoff;
+    float intensity;
+    bool active;
+};
+
+static_assert(sizeof(RenderCamera) == 28, "RenderCamera layout");
+static_assert(sizeof(LightDesc) == 40, "LightDesc layout");
+
+}
+
+namespace mb2 {
 
 // == render::InstanceData (include/madrona/render/ecs.hpp:49-63) + the instance's
 // world box (TLBVHNode in the reference)
 struct RenderInstance {
-    RVec3 position;
-    RQuat rotation;
-    RVec3 scale;
+    madrona::math::Vector3 position;
+    madrona::math::Quat rotation;
+    madrona::math::Vector3 scale;
     i32 matID;            // MaterialOverride: -1 mesh default, -2 use `color`, else material index
     i32 objectID;
     u32 color;            // 0xRRGGBB (ColorOverride)
@@ -28,8 +57,8 @@ struct RenderInstance {
 struct RenderLight {
     u32 directional;      // LightDesc::Type: true = Directional, false = Spotlight
     u32 castShadow;
-    RVec3 position;
-    RVec3 direction;
+    madrona::math::Vector3 position;
+    madrona::math::Vector3 direction;
     float cutoff;
     float intensity;
     u32 active;
@@ -39,8 +68,8 @@ constexpr int kMaxLightsPerWorld = 8;
 
 // == render::PerspectiveCameraData (include/madrona/render/ecs.hpp:38-46)
 struct RenderView {
-    RVec3 position;
-    RQuat rotation;       // inverse of the viewing entity's rotation
+    madrona::math::Vector3 position;
+    madrona::math::Quat rotation;       // inverse of the viewing entity's rotation
     float xScale;
     float yScale;
     float zNear;
@@ -50,16 +79,6 @@ struct RenderView {
 
 enum RenderCol : int { RCPosition = 0, RCRotation, RCScale, RCObjectID, RCRenderable, RCCount };
 
-// == the LightDesc component as the simulator's compiler lays it out
-struct LightDescComp {
-    unsigned char type;       // enum Type : bool
-    unsigned char castShadow;
-    float position[3];
-    float direction[3];
-    float cutoff;
-    float intensity;
-    unsigned char active;
-};
 constexpr int kMaxRenderArchetypes = 16;
 
 struct RenderArchetype {

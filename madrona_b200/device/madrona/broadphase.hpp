@@ -14,10 +14,6 @@
 #include <madrona/geo.hpp>
 #include <physics_state.h>
 
-namespace madrona::phys {
-struct ObjectManager;
-}
-
 namespace madrona::phys::broadphase {
 
 struct LeafID {
@@ -41,8 +37,7 @@ public:
 
     inline math::AABB getLeafAABB(LeafID leaf_id) const
     {
-        const mb2::PAABB &b = s_.leafAABBs[leaf_id.id];
-        return math::AABB { { b.pMin.x, b.pMin.y, b.pMin.z }, { b.pMax.x, b.pMax.y, b.pMax.z } };
+        return s_.leafAABBs[leaf_id.id];
     }
 
     template <typename Fn>

@@ -11,6 +11,9 @@
 // nodes, executed by the ahead-of-time sm_100a kernels in
 // csrc/kernels_physics.cu (candidates and contacts live in flat per-world
 // buffers, produced in deterministic order, so no Contact / Joint sorts).
+// The data-only layouts those kernels and the host asset builder read as well
+// (Velocity, JointConstraint, CollisionPrimitive, ObjectManager,
+// PhysicsSystemState, the xpbd per-body state ...) live in csrc/physics_state.h.
 #pragma once
 
 #include <madrona/math.hpp>
@@ -21,6 +24,7 @@
 
 #include <madrona/broadphase.hpp>
 #include <madrona/geo.hpp>
+#include <physics_state.h>
 
 namespace madrona::phys {
 
@@ -30,17 +34,6 @@ struct ExternalForce : math::Vector3 {
 
 struct ExternalTorque : math::Vector3 {
     inline ExternalTorque(math::Vector3 v) : Vector3(v) {}
-};
-
-enum class ResponseType : uint32_t {
-    Dynamic,
-    Kinematic,
-    Static,
-};
-
-struct Velocity {
-    math::Vector3 linear;
-    math::Vector3 angular;
 };
 
 struct SolverBundleAlias {};
@@ -70,38 +63,6 @@ struct ContactConstraint {
     math::Vector3 normal;
 };
 
-struct JointConstraint {
-    enum class Type {
-        Fixed,
-        Hinge
-    };
-
-    struct Fixed {
-        math::Quat attachRot1;
-        math::Quat attachRot2;
-        float separation;
-    };
-
-    struct Hinge {
-        math::Vector3 a1Local;
-        math::Vector3 a2Local;
-        math::Vector3 b1Local;
-        math::Vector3 b2Local;
-    };
-
-    Entity e1;
-    Entity e2;
-    Type type;
-
-    union {
-        Fixed fixed;
-        Hinge hinge;
-    };
-
-    math::Vector3 r1;
-    math::Vector3 r2;
-};
-
 struct CollisionEvent {
     Entity a;
     Entity b;
@@ -109,90 +70,11 @@ struct CollisionEvent {
 
 struct CollisionEventTemporary : Archetype<CollisionEvent> {};
 
-struct RigidBodyMassData {
-    float invMass;
-    math::Vector3 invInertiaTensor;
-    math::Vector3 toCenterOfMass;
-    math::Quat toInteriaFrame;
-};
-
-struct RigidBodyFrictionData {
-    float muS;
-    float muD;
-};
-
-struct RigidBodyMetadata {
-    RigidBodyMassData mass;
-    RigidBodyFrictionData friction;
-};
-
-struct CollisionPrimitive {
-    enum class Type : uint32_t {
-        Sphere = 1 << 0,
-        Hull = 1 << 1,
-        Plane = 1 << 2,
-    };
-
-    struct Sphere {
-        float radius;
-    };
-
-    struct Hull {
-        geo::HalfEdgeMesh halfEdgeMesh;
-    };
-
-    struct Plane {};
-
-    Type type;
-    union {
-        Sphere sphere;
-        Plane plane;
-        Hull hull;
-    };
-};
-
-struct ObjectManager {
-    CollisionPrimitive *collisionPrimitives;
-    math::AABB *primitiveAABBs;
-
-    math::AABB *rigidBodyAABBs;
-    uint32_t *rigidBodyPrimitiveOffsets;
-    uint32_t *rigidBodyPrimitiveCounts;
-    RigidBodyMetadata *metadata;
-};
-
 struct ObjectData {
     ObjectManager *mgr;
 };
 
-// == src/physics/physics_impl.hpp:7-15 (a singleton component, per world)
-struct PhysicsSystemState {
-    float deltaT;
-    float h;
-    math::Vector3 g;
-    float gMagnitude;
-    float restitutionThreshold;
-    uint32_t contactArchetypeID;
-    uint32_t jointArchetypeID;
-};
-
 namespace xpbd {
-
-// == src/physics/xpbd.cpp:26-46
-struct SubstepPrevState {
-    math::Vector3 prevPosition;
-    math::Quat prevRotation;
-};
-
-struct PreSolvePositional {
-    math::Vector3 x;
-    math::Quat q;
-};
-
-struct PreSolveVelocity {
-    math::Vector3 v;
-    math::Vector3 omega;
-};
 
 struct XPBDRigidBodyState : Bundle<
     SubstepPrevState,
@@ -322,7 +204,7 @@ inline void init(Context &ctx,
     bvh.leafEntities = (mb2::u64 *)carve(8 * max_leaves);
     bvh.objMgr = obj_mgr;
     bvh.leafObjIDs = (int32_t *)carve(4 * max_leaves);
-    bvh.leafAABBs = (mb2::PAABB *)carve(sizeof(mb2::PAABB) * max_leaves);
+    bvh.leafAABBs = (math::AABB *)carve(sizeof(math::AABB) * max_leaves);
     bvh.leafTransforms = (mb2::LeafTransform *)carve(sizeof(mb2::LeafTransform) * max_leaves);
     bvh.leafParents = (uint32_t *)carve(4 * max_leaves);
     bvh.sortedLeaves = (int32_t *)carve(4 * max_leaves);
@@ -361,7 +243,7 @@ inline broadphase::LeafID registerEntity(Context &ctx, Entity e, base::ObjectID 
     // tell the executor when spheres are in play (it then launches the narrowphase
     // variant that carries the sphere - hull path)
     {
-        const ObjectManager *obj_mgr = (const ObjectManager *)bvh.storage().objMgr;
+        const ObjectManager *obj_mgr = bvh.storage().objMgr;
         const uint32_t first = obj_mgr->rigidBodyPrimitiveOffsets[obj_id.idx];
         const uint32_t count = obj_mgr->rigidBodyPrimitiveCounts[obj_id.idx];
         for (uint32_t i = 0; i < count; i++) {
@@ -518,11 +400,11 @@ bool BVH::traceRayIntoLeaf(int32_t leaf_idx, math::Vector3 world_ray_o,
                            math::Vector3 world_ray_d, float t_min, float t_max,
                            float *hit_t, math::Vector3 *hit_normal)
 {
-    const ObjectManager *obj_mgr = (const ObjectManager *)s_.objMgr;
+    const ObjectManager *obj_mgr = s_.objMgr;
     const int32_t obj = s_.leafObjIDs[leaf_idx];
     const mb2::LeafTransform txfm = s_.leafTransforms[leaf_idx];
-    const math::Quat rot { txfm.rot.w, txfm.rot.x, txfm.rot.y, txfm.rot.z };
-    const math::Vector3 pos { txfm.pos.x, txfm.pos.y, txfm.pos.z };
+    const math::Quat rot = txfm.rot;
+    const math::Vector3 pos = txfm.pos;
     const math::Quat to_local = rot.inv();
 
     math::Vector3 obj_o = to_local.rotateVec(world_ray_o - pos);

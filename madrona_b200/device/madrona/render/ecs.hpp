@@ -3,7 +3,8 @@
 // RenderingSystem entry points; behind them the engine keeps flat per-world
 // instance / view arrays (filled by the render-prepare node) for the batch ray
 // caster in csrc/kernels_render.cu instead of the reference's render-entity
-// archetypes + three sorts per step.
+// archetypes + three sorts per step.  RenderCamera and LightDesc, which the
+// ray caster reads too, are defined in csrc/render_state.h.
 #pragma once
 
 #include <madrona/math.hpp>
@@ -13,34 +14,12 @@
 
 namespace madrona::render {
 
-struct RenderCamera {
-    Entity cameraEntity;      // the view's RaycastOutputArchetype entity
-    float fovScale;
-    float zNear;
-    math::Vector3 cameraOffset;
-};
-
 struct Renderable {
     Entity renderEntity;      // none() => not drawn
 };
 
 struct LightCarrier {
     Entity light;
-};
-
-// == include/madrona/render/ecs.hpp:65-115
-struct LightDesc {
-    enum Type : bool {
-        Directional = true,
-        Spotlight = false
-    };
-    Type type;
-    bool castShadow;
-    math::Vector3 position;
-    math::Vector3 direction;
-    float cutoff;
-    float intensity;
-    bool active;
 };
 
 struct LightDescDirection : math::Vector3 {

@@ -7,6 +7,5 @@ git stash -q
 make -C madrona_b200 -j8 > /dev/null
 cp madrona_b200/libmadrona_b200.so madrona_b200/libmadrona_b200_A.so
 git stash pop -q
-touch madrona_b200/csrc/*.cu madrona_b200/csrc/*.cpp
 make -C madrona_b200 -j8 > /dev/null
 ls -la madrona_b200/*.so
